@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- text GB/s scanned by the Boyer-Moore path on B200 (BASELINE.json's metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch of synthetic text:
@@ -17,6 +17,9 @@ One "step" = one pass of the hot path over one batch of synthetic text:
 `cpu_baseline`: the reference's own serial code (oracle/_ref/libref_bm.so, 1 core) on a bounded
            sample of the same text (rank 0, N = 1 only).
 --impl reference: the reference's own CPU code on all host threads (windowed), same metric.
+--dump-outputs DIR: what the last timed step returned (on rank 0: the match count and the ascending
+           start positions) as DIR/count.npy, DIR/positions.npy and DIR/positions_index.npy, float64.
+           The inputs are fixed by the workload's seeds, so two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -171,6 +174,26 @@ def verify_hits(torch, text, lo, pat, pos, count, cap):
     idx = (sample - lo).unsqueeze(1) + torch.arange(len(pat), device=text.device).unsqueeze(0)
     ok = ok and bool((text[idx] == pt.unsqueeze(0)).all().item())
     return ok
+
+
+DUMP_MAX_POSITIONS = 1 << 21     # positions + their indices, float64: 32 MiB per dump
+
+
+def dump_outputs(torch, out_dir, count, positions):
+    """Writes the result of one step as float64 arrays (exact for every position below 2^53): count.npy holds
+    the match count, positions.npy the ascending start positions and positions_index.npy their indices in
+    the full list.  A list longer than DUMP_MAX_POSITIONS is sampled at indices drawn from a fixed seed."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    held = 0 if positions is None else int(positions.numel())
+    idx = np.arange(held)
+    if held > DUMP_MAX_POSITIONS:
+        idx = np.sort(np.random.default_rng(0).choice(held, DUMP_MAX_POSITIONS, replace=False))
+        positions = positions[torch.from_numpy(idx).to(positions.device)]
+    vals = positions.cpu().numpy() if held else np.zeros(0)
+    np.save(out / "count.npy", np.array([count], dtype=np.float64))
+    np.save(out / "positions.npy", vals.astype(np.float64))
+    np.save(out / "positions_index.npy", idx.astype(np.float64))
 
 
 def oracle_lib():
@@ -524,6 +547,8 @@ def run_ours(args):
             total_hits, counts_all, gathered_list = state["last"]
             gathered_len = 0 if gathered_list is None else int(gathered_list.numel())
         ok = ok and total_hits == sum(counts_all) and counts_all[rank] == count
+    if args.dump_outputs and rank == 0:      # before the instrumented repeats below reuse the position buffer
+        dump_outputs(torch, args.dump_outputs, total_hits, gathered_list)
     ms_step = ms_total / args.steps
     value = total_n / (ms_step * 1e-3) / 1e9
 
@@ -791,7 +816,13 @@ def main():
     ap.add_argument("--no-balance", action="store_true", help="N > 1: skip the e2e leg with shards proportional to the ranks' ingest rates")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"], help="N > 1: exchange step over peer memory (library) or NCCL all-gather")
     ap.add_argument("--cpu-sample-bytes", type=int, default=4 * GIB)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the count and positions of the last timed step to DIR as .npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     # stdout carries exactly ONE JSON line: libraries that chat on fd 1 (NCCL's version banner)

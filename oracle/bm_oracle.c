@@ -293,6 +293,48 @@ int oracle_search_mt(const unsigned char *text, int64_t n, const unsigned char *
 }
 
 /* ------------------------------------------------------------------------------------------
+ * Harness: independent exact matcher (not reference code)
+ * ---------------------------------------------------------------------------------------- */
+
+/* Knuth-Morris-Pratt over the whole text.  Deliberately shares nothing with the Boyer-Moore
+ * restatement above or with the product's tables and filters: it is the truth those are
+ * checked against.  fail[j] = length of the longest proper border of pat[0..j]. */
+int oracle_kmp_search(const unsigned char *text, int64_t n, const unsigned char *pat, int32_t m,
+                      int64_t *pos, int64_t cap, uint64_t *count)
+{
+    if (m <= 0 || n < 0 || !count || (!text && n > 0) || !pat)
+        return -1;
+    int32_t *fail = (int32_t *)malloc(sizeof(int32_t) * (size_t)m);
+    if (!fail)
+        return -1;
+    fail[0] = 0;
+    for (int32_t j = 1, b = 0; j < m; ++j) {
+        while (b > 0 && pat[j] != pat[b])
+            b = fail[b - 1];
+        if (pat[j] == pat[b])
+            ++b;
+        fail[j] = b;
+    }
+    uint64_t found = 0;
+    int32_t q = 0;                           /* pattern bytes matched so far */
+    for (int64_t i = 0; i < n; ++i) {
+        while (q > 0 && text[i] != pat[q])
+            q = fail[q - 1];
+        if (text[i] == pat[q])
+            ++q;
+        if (q == m) {
+            if (pos && (int64_t)found < cap)
+                pos[found] = i - (m - 1);
+            ++found;
+            q = fail[m - 1];
+        }
+    }
+    *count = found;
+    free(fail);
+    return 0;
+}
+
+/* ------------------------------------------------------------------------------------------
  * Harness: synthetic text and position checksum
  * ---------------------------------------------------------------------------------------- */
 

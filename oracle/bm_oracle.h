@@ -72,6 +72,14 @@ void oracle_partition_words(const char *text_nul_terminated, int32_t P, int32_t 
 int oracle_search_mt(const unsigned char *text, int64_t n, const unsigned char *pat, int32_t m,
                      int64_t *pos, int64_t cap, uint64_t *count, int32_t nthreads);
 
+/* Independent exact matcher (harness, not reference code): Knuth-Morris-Pratt, linear time, all
+ * overlapping start positions ascending.  It shares no logic with the Boyer-Moore tables, the
+ * q-gram filters or the kernels, so the tests use it as the truth for both the restatement and
+ * the GPU path.  Writes up to cap positions into pos (may be NULL); *count is the full count.
+ * Returns 0, or -1 on bad args (m <= 0). */
+int oracle_kmp_search(const unsigned char *text, int64_t n, const unsigned char *pat, int32_t m,
+                      int64_t *pos, int64_t cap, uint64_t *count);
+
 /* Synthetic text shared by tests and bench (same definition as bmx_synth_fill_device):
  * 8 bytes per splitmix64 draw, word j = mix(seed + (j+1)*0x9E3779B97F4A7C15), byte k of the
  * draw b = (z >> 8k) & 0xFF is mapped to alphabet[(b * sigma) >> 8].  Fills text[0..len) with

@@ -1579,11 +1579,17 @@ int plan_scan(int device, int variant, int32_t m, bool positions, ScanArgs *a, S
     a->verify_smem = m <= kHaloSmemMax ? 1u : 0u;
     a->halo = a->verify_smem ? (uint32_t)((m + 15 + 15) & ~15) : 32u;
     a->pat_smem = (!multi && m <= kPatSmemMax) ? 1u : 0u;
-    a->stage_stride = (uint32_t)((kPre + tile + (int)a->halo + 127) & ~127);
 
     // 1 KiB per resident CTA is reserved by the driver.
     const size_t budget = std::min<size_t>((size_t)smem_optin, (size_t)smem_sm / ctas_per_sm - 1024);
-    int stages = (int)((budget - kCtlBytes - a->multi_smem) / a->stage_stride);
+    auto stages_for = [&](int t) {
+        a->stage_stride = (uint32_t)((kPre + t + (int)a->halo + 127) & ~127);
+        return (int)((budget - kCtlBytes - a->multi_smem) / a->stage_stride);
+    };
+    int stages = stages_for(tile);
+    // A 32 KiB tile next to the multi-pattern table and a halo for patterns of up to 4096 bytes leaves room for one
+    // stage only: such a set is scanned in 16 KiB tiles instead of failing.
+    if (stages < 2 && tile == 32768) stages = stages_for(tile = 16384);
     stages = std::min(stages, std::min(kMaxStages, env_int("BMX_STAGES", kMaxStages)));
     if (stages < 2) return fail(BMX_E_NOMEM, "pattern of %d bytes leaves room for %d pipeline stages", m, stages);
     a->stages = (uint32_t)stages;

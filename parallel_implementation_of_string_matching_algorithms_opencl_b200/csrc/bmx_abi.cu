@@ -137,9 +137,8 @@ int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
 
     const unsigned char *p = reinterpret_cast<const unsigned char *>(pat);
-    const char *knob_env = getenv("BMX_QGRAM_UNIFORM");
-    const int knob = (knob_env && *knob_env) ? atoi(knob_env) : -1;
-    if (s->d_block && s->m == m && s->requested_variant == variant && s->qgram_knob == knob && memcmp(s->pat.data(), p, (size_t)m) == 0) {
+    const Filter filter = choose_filter(variant, p, m);
+    if (s->d_block && s->m == m && s->filter == filter && memcmp(s->pat.data(), p, (size_t)m) == 0) {
         // same pattern as last time (a caller searching many texts for one pattern): tables and device block stand.
         // The upload was ordered on pat_stream only; any other stream waits for it (an event wait, no copy).
         if (st != s->pat_stream) BMX_CUDA(cudaStreamWaitEvent(st, s->ev_pat, 0));
@@ -147,9 +146,7 @@ int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t 
     }
     s->m = m;
     s->m_halo = 0;
-    s->requested_variant = variant;
-    s->qgram_knob = knob;
-    s->variant = resolve_variant(variant, m);
+    s->filter = filter;
     s->pat.assign(p, p + m);
 
     // Host image of the device block: tables once per pattern (BoyreMoore.cpp:153-190).
@@ -167,16 +164,13 @@ int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t 
         if (s->d_block) cudaFree(s->d_block);
         s->d_block = nullptr;
         s->d_block_cap = 0;
-        s->requested_variant = -1;
-        const int want_variant = variant;
         BMX_CUDA(cudaMalloc(&s->d_block, bytes));
-        s->requested_variant = want_variant;
         s->d_block_cap = bytes;
     }
     // pageable source: the runtime stages it before returning, so `image` may die afterwards
     const cudaError_t up = cudaMemcpyAsync(s->d_block, image.data(), bytes, cudaMemcpyHostToDevice, st);
     if (up != cudaSuccess) {
-        s->requested_variant = -1;   // nothing cached
+        s->m = 0;   // nothing cached: the block holds no whole pattern
         return fail(BMX_E_CUDA, "pattern upload: %s", cudaGetErrorString(up));
     }
     BMX_CUDA(cudaEventRecord(s->ev_pat, st));
@@ -187,7 +181,7 @@ int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t 
     s->proto.g_bad = reinterpret_cast<const int32_t *>(s->d_block);
     s->proto.g_good = reinterpret_cast<const int32_t *>(static_cast<unsigned char *>(s->d_block) + good_off);
     s->proto.g_pat = static_cast<const uint8_t *>(s->d_block) + pat_off;
-    fill_filter_constants(s->variant, p, m, &s->proto);
+    fill_filter_constants(filter, p, m, &s->proto);
     return BMX_OK;
 }
 
@@ -203,7 +197,7 @@ int bmx_scanner_begin(bmx_scanner *s, int64_t *d_pos_out, int64_t pos_cap, void 
     s->find_epoch = 0;
     s->timing_open = false;
     s->stats = bmx_stats{};
-    s->stats.variant = s->variant;
+    s->stats.variant = s->m > 0 ? filter_variant(s->filter) : BMX_VARIANT_AUTO;
     // no device work here: the first scan of the search treats the carried state as zero (ScanArgs::first_scan)
     (void)stream;
     return BMX_OK;
@@ -229,7 +223,7 @@ int bmx_scanner_scan(bmx_scanner *s, const void *d_text, int64_t n, int64_t pos_
     a.pos_cap = s->pos_cap;
 
     ScanLaunch launch{};
-    if (int rc = plan_scan(s->device, s->variant, s->m_halo ? s->m_halo : s->m, s->positions, &a, &launch)) return rc;
+    if (int rc = plan_scan(s->device, s->filter, s->m_halo ? s->m_halo : s->m, s->positions, &a, &launch)) return rc;
 
     // scratch: two "zero halves" [tickets 16 B | scan count u64 + pad | block_sum u32 x blocks | seg_count u16 x segs |
     //          item_flag u8 x items], each zero whenever a scan starts on it, followed by

@@ -34,11 +34,49 @@ constexpr int kSegBytes = 2048;
 constexpr int kSegChunks = kSegBytes / 16;   // 128
 constexpr int kBlockSegs = 1024;
 constexpr int64_t kBlockBytes = (int64_t)kSegBytes * kBlockSegs;   // 2 MiB
+
 // A block is "dense" from this many hits on (6 % of its start positions): its items are then expanded in
 // ticket order by whole CTAs, which keeps the write frontier narrow (profiles/micro/write_patterns.cu).
 constexpr uint32_t kDenseBlockHits = 1u << 17;
 constexpr int kExpandSplit = 64;                      // expand work items per block
 constexpr int kItemSegs = kBlockSegs / kExpandSplit;  // 16 segments = 32 KiB of text, one warp each
+
+// The scan kernel's filter kinds: one scan_kernel family each.  choose_filter() (bmx_scan.cu) picks one per pattern;
+// the kernel, its constants and its launch plan all follow from that one value.
+enum Filter : int {
+    kQgramPerResidue,   // QGRAM, 7 <= m <= 10: one hash multiplier per residue (m <= 9 on small alphabets unless forced)
+    kQgram,             // QGRAM: one hash multiplier for all four residues
+    kWindow4,           // WINDOW, m >= 4: the 4-byte window at every position against P[0..4)
+    kBytes1,            // WINDOW, m = 1, 2, 3: all m bytes at four start positions per word at once
+    kBytes2,
+    kBytes3,
+    kBytes5,            // WINDOW, m = 5, 6 on small alphabets: the first five bytes, four start positions per word
+    kShiftAnd,          // SHIFTAND, m <= 32
+    kMulti,             // a multi-pattern set (bmx_multipat.cu)
+    kFilterCount
+};
+
+// The public bmx_variant a kind belongs to (kMulti belongs to none: AUTO).
+constexpr __host__ __device__ int filter_variant(Filter f)
+{
+    if (f == kQgramPerResidue || f == kQgram) return BMX_VARIANT_QGRAM;
+    if (f == kWindow4 || f == kBytes1 || f == kBytes2 || f == kBytes3 || f == kBytes5) return BMX_VARIANT_WINDOW;
+    return f == kShiftAnd ? BMX_VARIANT_SHIFTAND : BMX_VARIANT_AUTO;
+}
+// Start position of mask bit 0 relative to its 16-byte chunk: the q-gram hashes flag starts up to 3 bytes in front.
+constexpr __host__ __device__ int filter_owner_offset(Filter f) { return f == kQgramPerResidue || f == kQgram || f == kMulti ? -3 : 0; }
+// Pattern bytes a byte-parallel kind tests (0: not byte-parallel).
+constexpr __host__ __device__ int filter_bytes(Filter f)
+{
+    return f == kBytes1 ? 1 : f == kBytes2 ? 2 : f == kBytes3 ? 3 : f == kBytes5 ? 5 : 0;
+}
+// Kinds whose filter is exact for every pattern they run: no candidate is ever verified.
+constexpr __host__ __device__ bool filter_never_verifies(Filter f) { return f == kShiftAnd || f == kBytes1 || f == kBytes2 || f == kBytes3; }
+// The filter's candidates are the matches of an m-byte pattern: nothing to verify.
+constexpr __host__ __device__ bool filter_exact(Filter f, int32_t m)
+{
+    return f == kShiftAnd || (filter_variant(f) == BMX_VARIANT_WINDOW && (m <= 4 || (f == kBytes5 && m == 5)));
+}
 
 // Kernel arguments (passed by value: they live in the constant bank of the launch).
 struct ScanArgs {
@@ -60,10 +98,10 @@ struct ScanArgs {
     uint32_t f[4];          // QGRAM: hash of P[r..r+q) for r = 0..3; WINDOW: f[0] = target
     uint32_t hmul;          // QGRAM: hash multiplier K << (32 - 8*(q-4)); the shift drops the bytes beyond the q-gram
     uint32_t hmulr[4];      // QGRAM, 7 <= m <= 10: one multiplier per residue (residue r sees min(8, m - r) bytes)
-    uint32_t mulc;          // WINDOW: 2^(32-8q), drops the bytes beyond q
+    uint32_t pad0;          // pad0, pad1: bcast and every field behind it stay at the offsets the kernels were tuned with;
+                            // shifted, the byte-parallel kernels lost 0.5-0.8 % count-only (NVIDIA B200, 1000 W power limit)
     uint32_t bcast[5];      // WINDOW, byte-parallel kernels: pattern byte k replicated into the four bytes of a word
-    uint32_t pat_distinct;  // distinct byte values among the pattern's first 16 bytes (the only hint of the text's alphabet)
-    uint32_t window5;       // WINDOW, m = 5, 6 on small alphabets: byte-parallel test of the first five bytes (plan_scan)
+    uint32_t pad1[2];
     // per-pattern block in global memory
     const uint8_t *g_pat;
     const int32_t *g_bad;
@@ -107,26 +145,24 @@ struct ScanArgs {
 
 // Launch description produced by plan_scan() and consumed by launch_scan().
 struct ScanLaunch {
-    int variant;        // resolved bmx_variant
+    Filter filter;
     int tile_bytes;
     int grid;
     size_t smem_bytes;
 };
 
 // Host entry points implemented in bmx_scan.cu.
-int resolve_variant(int requested, int32_t m);
-int plan_scan(int device, int variant, int32_t m, bool positions, ScanArgs *args, ScanLaunch *out);
+Filter choose_filter(int requested_variant, const unsigned char *pat, int32_t m);
+int plan_scan(int device, Filter filter, int32_t m, bool positions, ScanArgs *args, ScanLaunch *out);
 int launch_scan(const ScanArgs &args, const ScanLaunch &launch, bool positions, void *stream);
 int launch_emit(const ScanArgs &args, void *stream);
 int launch_export_result(const unsigned long long *d_count, const int64_t *d_pos, int64_t pos_cap, void *d_dst, int64_t head,
                          void *stream);   // block-scan + expand (positions mode)
 int launch_synth_fill(void *d_text, int64_t offset, int64_t len, uint64_t seed,
                       const unsigned char *alphabet, int32_t sigma, void *stream);
-int launch_partition_count(const int64_t *d_pos, const unsigned long long *d_count, int64_t pos_cap,
-                           const int32_t *d_se, int32_t *d_ans, int32_t m, int32_t nparts, void *stream);
 
-// Filter constants for a pattern (host).
-void fill_filter_constants(int variant, const unsigned char *pat, int32_t m, ScanArgs *args);
+// Filter constants of a single-pattern kind (host).
+void fill_filter_constants(Filter filter, const unsigned char *pat, int32_t m, ScanArgs *args);
 
 constexpr uint32_t kHashMul = 0x9E3779B1u;
 // multi-pattern candidate table
@@ -138,7 +174,6 @@ constexpr int kMultiSlots = 1 << kMultiSlotsLog2;
 constexpr uint32_t kMultiSlotMul = 0x85EBCA6Bu;
 constexpr uint32_t kHashMul2 = 0xC2B2AE3Du;
 constexpr size_t kMultiSmemBytes = (size_t)kMultiBitmapWords * 4 + (size_t)kMultiSlots * 8 + (size_t)kMultiMaxPatterns * 8;
-constexpr int BMX_VARIANT_MULTI_INTERNAL = 4;                          // not part of the public bmx_variant enum
 constexpr unsigned long long kFindMask = (1ull << 47) - 1;   // find-first keys: positions below 2^47
 
 }  // namespace bmx

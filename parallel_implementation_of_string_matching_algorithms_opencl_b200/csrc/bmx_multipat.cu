@@ -171,7 +171,7 @@ int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, in
 
     bmx_scanner *s = c.scanner;
     // the scanner leaves single-pattern mode: its cached pattern block no longer describes proto
-    s->requested_variant = -1;
+    s->filter = kMulti;
     s->pat.clear();
     s->proto = ScanArgs{};
     s->proto.m = im.m_min;
@@ -187,7 +187,6 @@ int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, in
     s->proto.multi_blob_smem = blob_bytes <= (size_t)kPatSmemMax * 4 ? (uint32_t)blob_bytes : 0u;   // SmemCtl::good holds kPatSmemMax ints
     s->m = im.m_min;
     s->m_halo = im.m_max;
-    s->variant = BMX_VARIANT_MULTI_INTERNAL;
     const int keep_timing = s->timing_level;
     s->timing_level = 0;
 
@@ -227,7 +226,6 @@ int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, in
     }
     s->timing_level = keep_timing;
     s->m_halo = 0;
-    s->variant = 0;
     s->m = 0;   // the scanner has no single pattern until the next set_pattern
     if (rc != BMX_OK) return rc;
     for (int32_t k = 0; k < npat; ++k) counts[k] = h_counts[(size_t)k];

@@ -300,8 +300,6 @@ __device__ __forceinline__ uint32_t valid_bits(int64_t p0, int64_t vmin, int64_t
 // ---------------------------------------------------------------------------------------------
 // The scan kernel
 // ---------------------------------------------------------------------------------------------
-enum : int { kQgram = 1, kWindow = 2, kShiftAnd = 3, kMulti = 4 };
-
 // WINDOW: the 4-byte window that starts s bytes into `lo` (continuing in `hi`).  (Building the
 // shifted windows on the FMA pipe with IMAD.HI/IMAD instead of SHF was measured 13 % slower.)
 __device__ __forceinline__ uint32_t window_at(uint32_t lo, uint32_t hi, int s)
@@ -325,16 +323,14 @@ __device__ __forceinline__ uint32_t window_flags(uint32_t lo, uint32_t hi, uint3
     return ~(a | z) & 0x80808080u;
 }
 
-// FLAG: QGRAM -> 1: one hash multiplier for all four residues, 0: one per residue (7 <= m <= 10).
-//       WINDOW -> 1: whole 4-byte windows (m >= 4); 2, 3, 4: m = 1, 2, 3 (byte-parallel flags, window_flags<m>).
-template <int VARIANT, int FLAG>
+template <Filter F>
 __device__ __forceinline__ bool filter_any(const uint4 &w, uint32_t w4, const ScanArgs &A)
 {
-    if (VARIANT == kQgram) {
+    if (filter_variant(F) == BMX_VARIANT_QGRAM) {
         const uint32_t f0 = A.f[0], f1 = A.f[1], f2 = A.f[2], f3 = A.f[3];
         // hmul = K << (32 - 8*q2): the multiplication itself drops the bytes of the second word that lie
         // beyond the q-gram (7 <= m <= 10), so short patterns need no masking instruction
-        if (!FLAG) {
+        if (F == kQgramPerResidue) {
             // 7 <= m <= 10: residue r may use min(8, m - r) pattern bytes, so each residue hashes with its
             // own multiplier -- 3 more IMADs per word, several times fewer candidates on small alphabets
             const uint32_t k0 = A.hmulr[0], k1 = A.hmulr[1], k2 = A.hmulr[2], k3 = A.hmulr[3];
@@ -358,8 +354,8 @@ __device__ __forceinline__ bool filter_any(const uint4 &w, uint32_t w4, const Sc
         any |= (h3 == f0) | (h3 == f1) | (h3 == f2) | (h3 == f3);
         return any;
     } else {
-        if (FLAG >= 2) {   // m = FLAG - 1 <= 3, or (FLAG 6) the first five bytes of a 5- or 6-byte pattern
-            constexpr int M = FLAG == 6 ? 5 : (FLAG >= 2 ? FLAG - 1 : 1);
+        if constexpr (filter_bytes(F) != 0) {   // m <= 3, or the first five bytes of a 5- or 6-byte pattern
+            constexpr int M = filter_bytes(F);
             const uint32_t b0 = A.bcast[0], b1 = A.bcast[1], b2 = A.bcast[2], b3 = A.bcast[3], b4 = A.bcast[4];
             return (window_flags<M>(w.x, w.y, b0, b1, b2, b3, b4) | window_flags<M>(w.y, w.z, b0, b1, b2, b3, b4) |
                     window_flags<M>(w.z, w.w, b0, b1, b2, b3, b4) | window_flags<M>(w.w, w4, b0, b1, b2, b3, b4)) != 0u;
@@ -376,26 +372,26 @@ __device__ __forceinline__ bool filter_any(const uint4 &w, uint32_t w4, const Sc
     }
 }
 
-template <int VARIANT, int FLAG>
+template <Filter F>
 __device__ __forceinline__ uint32_t filter_mask(const uint4 &w, uint32_t w4, const ScanArgs &A)
 {
     uint32_t mask = 0;
     const uint32_t ww[5] = {w.x, w.y, w.z, w.w, w4};
-    if (VARIANT == kQgram) {
+    if (filter_variant(F) == BMX_VARIANT_QGRAM) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const uint32_t h = ww[j] + A.hmul * ww[j + 1];
             // word j with residue r flags start position 4j - r, i.e. bit 4j + 3 - r (bit 0 = c - 3)
 #pragma unroll
             for (int r = 0; r < 4; ++r) {
-                const uint32_t hr = FLAG ? h : ww[j] + A.hmulr[r] * ww[j + 1];
+                const uint32_t hr = F == kQgram ? h : ww[j] + A.hmulr[r] * ww[j + 1];
                 mask |= (uint32_t)(hr == A.f[r]) << (4 * j + 3 - r);
             }
         }
-    } else if (FLAG >= 2) {
-        // m = FLAG - 1 <= 3: flags of two words share one multiply that gathers their eight 0x80 bits into one byte
+    } else if constexpr (filter_bytes(F) != 0) {
+        // flags of two words share one multiply that gathers their eight 0x80 bits into one byte
         // ((c0 >> 4 | c1) * 0x204081 >> 24: bits 3,11,19,27 and 7,15,23,31 land on 24..31 in position order, no carries)
-        constexpr int M = FLAG == 6 ? 5 : (FLAG >= 2 ? FLAG - 1 : 1);
+        constexpr int M = filter_bytes(F);
         const uint32_t b0 = A.bcast[0], b1 = A.bcast[1], b2 = A.bcast[2], b3 = A.bcast[3], b4 = A.bcast[4];
         const uint32_t c0 = window_flags<M>(ww[0], ww[1], b0, b1, b2, b3, b4), c1 = window_flags<M>(ww[1], ww[2], b0, b1, b2, b3, b4);
         const uint32_t c2 = window_flags<M>(ww[2], ww[3], b0, b1, b2, b3, b4), c3 = window_flags<M>(ww[3], ww[4], b0, b1, b2, b3, b4);
@@ -582,12 +578,12 @@ struct VerifyCtx {
 // a tile without the any-pass and the vote -- every lane builds its masks right away.  Kept out of
 // line so the common path of scan_kernel stays exactly the sparse filter loop.  Returns the hits
 // found (count-only mode adds them up) with bit 63 set while the text is still dense.
-template <int VARIANT, int FLAG, int TILE, bool POSITIONS>
+template <Filter F, int TILE, bool POSITIONS>
 __device__ __forceinline__ unsigned long long dense_tile_body(const ScanArgs &A, const uint8_t *st, int64_t tile_v0,
                                                               VerifyCtx vc, int warp, int lane)
 {
     constexpr int WARP_BYTES = TILE / kConsumerWarps;
-    constexpr int OFFS = (VARIANT == kQgram || VARIANT == kMulti) ? -3 : 0;
+    constexpr int OFFS = filter_owner_offset(F);
     unsigned long long found = 0;
     uint32_t cand_lanes = 0, tile_total = 0;
     const uint32_t tile_seg0 = (uint32_t)(tile_v0 / kSegBytes);   // 32-bit segment index of the tile's first segment
@@ -602,7 +598,7 @@ __device__ __forceinline__ unsigned long long dense_tile_body(const ScanArgs &A,
         unsigned long long cand64 = 0;
 #pragma unroll
         for (int sl = 0; sl < 4; ++sl) {
-            uint32_t cand = filter_mask<VARIANT, FLAG>(w[sl], w4[sl], A);
+            uint32_t cand = filter_mask<F>(w[sl], w4[sl], A);
             if (!vc.all_valid) cand &= valid_bits(seg_p0 + sl * 512, A.vmin, A.vmax);
             cand64 |= (unsigned long long)cand << (16 * sl);
         }
@@ -626,24 +622,24 @@ __device__ __forceinline__ unsigned long long dense_tile_body(const ScanArgs &A,
 // out of line the kernel arguments are reached through a generic pointer (LD.E, a long-scoreboard stall per segment:
 // profiles/r02_ncu_scan_eng_is.txt), inline they are constant-bank operands ('is' on English prose count-only 4.52 ->
 // 4.86 TB/s, ' ' 5.25 -> 5.78).  m = 3 stays out of line: inlined, its SPARSE path lost 7 % (bytes256: 6.6 -> 5.95 TB/s).
-template <int VARIANT, int FLAG, int TILE, bool POSITIONS>
+template <Filter F, int TILE, bool POSITIONS>
 __device__ __noinline__ unsigned long long dense_tile(const ScanArgs &A, const uint8_t *st, int64_t tile_v0, VerifyCtx vc, int warp, int lane)
 {
-    return dense_tile_body<VARIANT, FLAG, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
+    return dense_tile_body<F, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
 }
 
-template <int VARIANT, int FULL8, int TILE, bool POSITIONS>
+template <Filter F, int TILE, bool POSITIONS>
 __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant__ ScanArgs A)
 {
     constexpr int WARP_BYTES = TILE / kConsumerWarps;   // contiguous bytes owned by one warp
-    constexpr int OFFS = (VARIANT == kQgram || VARIANT == kMulti) ? -3 : 0;    // start position of bit 0 relative to the chunk
+    constexpr int OFFS = filter_owner_offset(F);        // start position of bit 0 relative to the chunk
     constexpr int SEGS = WARP_BYTES / kSegBytes;        // 2 KiB segments per warp per tile
     static_assert(SEGS >= 1 && SEGS * kSegBytes * kConsumerWarps == TILE, "tile must be a multiple of 16 KiB");
-    constexpr int kSegUnroll = (VARIANT == kWindow && FULL8 == 1) ? 1 : SEGS;
+    constexpr int kSegUnroll = F == kWindow4 ? 1 : SEGS;
 
     extern __shared__ __align__(128) uint8_t smem[];
     SmemCtl *ctl = reinterpret_cast<SmemCtl *>(smem);
-    uint8_t *stages = smem + kCtlBytes + (VARIANT == kMulti ? A.multi_smem : 0u);
+    uint8_t *stages = smem + kCtlBytes + (F == kMulti ? A.multi_smem : 0u);
 
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
@@ -653,7 +649,7 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
     M.bits = reinterpret_cast<const uint32_t *>(smem + kCtlBytes);
     M.table = reinterpret_cast<const uint2 *>(smem + kCtlBytes + (size_t)kMultiBitmapWords * 4);
     M.dir = reinterpret_cast<const uint2 *>(smem + kCtlBytes + (size_t)kMultiBitmapWords * 4 + (size_t)kMultiSlots * 8);
-    const uint8_t *mblob = (VARIANT == kMulti && A.multi_blob_smem) ? reinterpret_cast<const uint8_t *>(ctl->good) : A.g_mblob;
+    const uint8_t *mblob = (F == kMulti && A.multi_blob_smem) ? reinterpret_cast<const uint8_t *>(ctl->good) : A.g_mblob;
 
     // Fetches one tile (plus the 16 bytes in front of it and the halo behind it) into pipeline slot s.
     auto fetch_tile = [&](uint32_t tile, uint32_t s) {
@@ -704,10 +700,10 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
             ctl->rpat[i] = (uint32_t)q[0] | ((uint32_t)q[1] << 8) | ((uint32_t)q[2] << 16) | ((uint32_t)q[3] << 24);
         }
     }
-    if (VARIANT == kShiftAnd) {
+    if (F == kShiftAnd) {
         for (int i = tid; i < 256; i += kThreads) ctl->sa_mask[i] = 0u;
     }
-    if (VARIANT == kMulti) {
+    if (F == kMulti) {
         uint4 *dst = reinterpret_cast<uint4 *>(smem + kCtlBytes);
         const uint4 *b4 = reinterpret_cast<const uint4 *>(A.g_mbits), *t4 = reinterpret_cast<const uint4 *>(A.g_mtable),
                     *d4 = reinterpret_cast<const uint4 *>(A.g_mdir);
@@ -722,7 +718,7 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
         }
     }
     __syncthreads();
-    if (VARIANT == kShiftAnd) {
+    if (F == kShiftAnd) {
         for (int i = tid; i < A.m; i += kThreads) atomicOr(&ctl->sa_mask[A.g_pat[i]], 1u << i);
         __syncthreads();
     }
@@ -757,10 +753,11 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
     const int32_t *bad = A.pat_smem ? ctl->bad : A.g_bad;
     const int32_t *good = A.pat_smem ? ctl->good : A.g_good;
     const uint32_t *rpat = A.pat_smem ? ctl->rpat : nullptr;
-    const bool exact_filter = (VARIANT == kShiftAnd) || (VARIANT == kWindow && (A.m <= 4 || (FULL8 == 6 && A.m == 5)));
+    // (m decides only for the WINDOW kinds: the others pass a constant, so the call folds in the front end and the
+    // out-of-line dense_tile is compiled knowing the value)
+    const bool exact_filter = filter_exact(F, filter_variant(F) == BMX_VARIANT_WINDOW ? A.m : 0);
     // flagged chunks are checked by the whole warp when pattern and window both sit in shared memory (m <= kPatSmemMax)
-    constexpr bool kNeverVerifies = (VARIANT == kShiftAnd) || (VARIANT == kWindow && FULL8 >= 2 && FULL8 <= 4);   // m <= 3: the filter is exact
-    const bool coop = !kNeverVerifies && !exact_filter && A.pat_smem != 0u && A.verify_smem != 0u && A.coop_verify != 0u;
+    const bool coop = !filter_never_verifies(F) && !exact_filter && A.pat_smem != 0u && A.verify_smem != 0u && A.coop_verify != 0u;
     const uint32_t *patw = reinterpret_cast<const uint32_t *>(ctl->pat);
     CoopLane cl{};
     if (coop) cl = coop_lane_setup<OFFS>(patw, A.m, lane);
@@ -780,12 +777,12 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
         const bool all_valid = tile_v0 + OFFS >= A.vmin && tile_v0 + (TILE - 1) + OFFS <= A.vmax;
 
         bool took_dense = false;
-        if constexpr (VARIANT != kShiftAnd && VARIANT != kMulti) {
+        if constexpr (F != kShiftAnd && F != kMulti) {
             if (dense_mode) {
                 const VerifyCtx vc{vbase, pat, rpat, bad, good, exact_filter, all_valid};
                 unsigned long long r;
-                if constexpr (VARIANT == kWindow && (FULL8 == 2 || FULL8 == 3)) r = dense_tile_body<VARIANT, FULL8, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
-                else r = dense_tile<VARIANT, FULL8, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
+                if constexpr (F == kBytes1 || F == kBytes2) r = dense_tile_body<F, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
+                else r = dense_tile<F, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
                 dense_mode = (r >> 63) != 0;
                 if (!POSITIONS) my_count += r & ~(1ull << 63);
                 took_dense = true;
@@ -802,7 +799,7 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
                 const uint32_t seg_off = warp * WARP_BYTES + sg * kSegBytes;   // this warp's 2 KiB segment
                 const int64_t seg_p0 = tile_v0 + seg_off + lane * 16 + OFFS;   // start position of bit 0, slab 0
                 bool has_hits = false;
-                if (VARIANT == kShiftAnd) {
+                if (F == kShiftAnd) {
 #pragma unroll
                     for (int sl = 0; sl < 4; ++sl) {
                         uint32_t hits = shiftand_chunk(st + seg_off + sl * 512 + lane * 16, A.m, ctl->sa_mask);
@@ -816,14 +813,14 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
                     uint32_t w4[4];
                     load_segment(st + seg_off, lane, w, w4);
                     uint32_t w5[4] = {0u, 0u, 0u, 0u};
-                    if (VARIANT == kMulti && A.hmul2 != 0u) load_second_after(st + seg_off, lane, w, w5);
+                    if (F == kMulti && A.hmul2 != 0u) load_second_after(st + seg_off, lane, w, w5);
                     bool any[4];
 #pragma unroll
                     for (int sl = 0; sl < 4; ++sl)
-                        any[sl] = VARIANT == kMulti ? multi_any(w[sl], w4[sl], w5[sl], A.hmul, A.hmul2, M.bits) : filter_any<VARIANT, FULL8>(w[sl], w4[sl], A);
+                        any[sl] = F == kMulti ? multi_any(w[sl], w4[sl], w5[sl], A.hmul, A.hmul2, M.bits) : filter_any<F>(w[sl], w4[sl], A);
                     const uint32_t vote = __ballot_sync(0xFFFFFFFFu, any[0] | any[1] | any[2] | any[3]);
                     if (vote) {  // warp-uniform and rare: the common path ends at this branch
-                        if (VARIANT == kMulti) {
+                        if (F == kMulti) {
 #pragma unroll
                             for (int sl = 0; sl < 4; ++sl) {
                                 if (any[sl]) {
@@ -851,7 +848,7 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
                             for (int sl = 0; sl < 4; ++sl) {
                                 if (any[sl]) {
                                     const int64_t p0 = seg_p0 + sl * 512;
-                                    uint32_t cand = filter_mask<VARIANT, FULL8>(w[sl], w4[sl], A);
+                                    uint32_t cand = filter_mask<F>(w[sl], w4[sl], A);
                                     if (!all_valid) cand &= valid_bits(p0, A.vmin, A.vmax);
                                     if (cand)
                                         hm[sl] = exact_filter ? cand : (uint32_t)verify_candidates(cand, vbase, p0, A.m, pat, rpat, bad, good, A.verify_smem != 0);
@@ -1384,49 +1381,13 @@ __global__ void export_result_kernel(const unsigned long long *count, const int6
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) dst[2 + i] = pos[i];
 }
 
-// ans[id] = number of positions p with se[2id] <= p and p + m - 1 <= se[2id+1]
-// (occurrences lying fully inside the inclusive range, kernel1.cl:15,19).
-__global__ void partition_count_kernel(const int64_t *pos, const unsigned long long *count, int64_t pos_cap,
-                                       const int32_t *se, int32_t *ans, int32_t m, int32_t nparts)
-{
-    const int id = blockIdx.x * blockDim.x + threadIdx.x;
-    if (id >= nparts) return;
-    int64_t n = (int64_t)*count;
-    if (n > pos_cap) n = pos_cap;
-    const int64_t lo_v = se[2 * id], hi_v = (int64_t)se[2 * id + 1] - (m - 1);
-    int64_t a = 0, b = n;  // first index with pos >= lo_v
-    while (a < b) {
-        const int64_t mid = (a + b) >> 1;
-        if (pos[mid] < lo_v) a = mid + 1; else b = mid;
-    }
-    const int64_t first = a;
-    a = first, b = n;  // first index with pos > hi_v
-    while (a < b) {
-        const int64_t mid = (a + b) >> 1;
-        if (pos[mid] <= hi_v) a = mid + 1; else b = mid;
-    }
-    ans[id] = (int32_t)(a > first ? a - first : 0);
-}
-
 // ---------------------------------------------------------------------------------------------
-// Host: variant choice, planning, launch
+// Host: filter choice, planning, launch
 // ---------------------------------------------------------------------------------------------
 static int env_int(const char *name, int fallback)
 {
     const char *v = getenv(name);
     return (v && *v) ? atoi(v) : fallback;
-}
-
-int resolve_variant(int requested, int32_t m)
-{
-    switch (requested) {
-    case BMX_VARIANT_QGRAM: return m >= 7 ? BMX_VARIANT_QGRAM : BMX_VARIANT_WINDOW;
-    case BMX_VARIANT_WINDOW: return BMX_VARIANT_WINDOW;
-    case BMX_VARIANT_SHIFTAND: return m <= 32 ? BMX_VARIANT_SHIFTAND : BMX_VARIANT_QGRAM;
-    default: break;
-    }
-    // AUTO: thresholds from the measured table in DESIGN.md (profiles/variants_r01.json).
-    return m >= 7 ? BMX_VARIANT_QGRAM : BMX_VARIANT_WINDOW;
 }
 
 static uint32_t le_word(const unsigned char *p, int nbytes)
@@ -1436,94 +1397,77 @@ static uint32_t le_word(const unsigned char *p, int nbytes)
     return w;
 }
 
-void fill_filter_constants(int variant, const unsigned char *pat, int32_t m, ScanArgs *a)
+Filter choose_filter(int requested_variant, const unsigned char *pat, int32_t m)
 {
-    {
-        bool seen[256] = {false};
-        uint32_t distinct = 0;
-        for (int i = 0; i < m && i < 16; ++i)
-            if (!seen[pat[i]]) { seen[pat[i]] = true; ++distinct; }
-        a->pat_distinct = distinct;
+    // AUTO, and QGRAM for m < 7: thresholds from the measured table in DESIGN.md (profiles/variants_r01.json)
+    int variant = m >= 7 ? BMX_VARIANT_QGRAM : BMX_VARIANT_WINDOW;
+    if (requested_variant == BMX_VARIANT_WINDOW) variant = BMX_VARIANT_WINDOW;
+    if (requested_variant == BMX_VARIANT_SHIFTAND) variant = m <= 32 ? BMX_VARIANT_SHIFTAND : BMX_VARIANT_QGRAM;
+    if (variant == BMX_VARIANT_SHIFTAND) return kShiftAnd;
+    // The text's alphabet is unknown here; the distinct bytes among the pattern's first 16 are the proxy.
+    bool seen[256] = {false};
+    int distinct = 0;
+    for (int i = 0; i < m && i < 16; ++i)
+        if (!seen[pat[i]]) { seen[pat[i]] = true; ++distinct; }
+    if (variant == BMX_VARIANT_QGRAM) {
+        // Per-residue lengths cost 3 more IMADs per word: measured -6 % on large alphabets, where the
+        // shortest length is selective enough anyway, and +35 % / +32 % / +11 % on 4-letter text at m = 7 / 8 /
+        // 9 (profiles/short_qgram_r01.txt).
+        const int knob = env_int("BMX_QGRAM_UNIFORM", -1);   // measurement knob: 1 / 0 force one / four lengths
+        const bool per_residue = knob >= 0 ? knob == 0 : (m <= 9 && distinct <= 4);
+        return per_residue && m <= 10 ? kQgramPerResidue : kQgram;   // from m = 11 on every residue sees 8 bytes
     }
+    if (m <= 3) return m == 1 ? kBytes1 : (m == 2 ? kBytes2 : kBytes3);
+    // m = 5, 6: the 4-byte window passes 1 in 256 positions of a 4-letter text and the scan becomes
+    // verification-bound (DNA: 2.0 / 2.2 TB/s).  The byte-parallel construction of the m <= 3 kernels, extended to five
+    // bytes (11 instructions per word instead of 7, exact for m = 5), is chosen when the pattern has <= 4 distinct
+    // bytes -- the same proxy as in the q-gram layout choice.  BMX_WINDOW5=0/1 forces either.
+    if ((m == 5 || m == 6) && env_int("BMX_WINDOW5", distinct <= 4 ? 1 : 0) != 0) return kBytes5;
+    return kWindow4;
+}
+
+void fill_filter_constants(Filter filter, const unsigned char *pat, int32_t m, ScanArgs *a)
+{
     a->f[0] = a->f[1] = a->f[2] = a->f[3] = 0;
     a->hmul = kHashMul;
-    a->mulc = 1u;
-    if (variant == BMX_VARIANT_QGRAM) {
-        // residue r (pattern byte r on a word boundary) can use min(8, m - r) pattern bytes; for m >= 11
-        // that is 8 for every residue and one multiplier serves all four (a->hmul, the FULL8 kernels)
+    if (filter_variant(filter) == BMX_VARIANT_QGRAM) {
+        // residue r (pattern byte r on a word boundary) can use min(8, m - r) pattern bytes
         for (int r = 0; r < 4; ++r) {
             const int q2 = std::min(m - r, 8) - 4;   // bytes taken from the second word
             a->hmulr[r] = q2 >= 4 ? kHashMul : (q2 == 0 ? 0u : (kHashMul << (32 - 8 * q2)));
             a->f[r] = le_word(pat + r, 4) + a->hmulr[r] * le_word(pat + r + 4, q2);
         }
         a->hmul = a->hmulr[3];
-        // Per-residue lengths cost 3 more IMADs per word: measured -6 % on large alphabets, where the
-        // shortest length is selective enough anyway, and +35 % / +32 % / +11 % on 4-letter text at m = 7 / 8 /
-        // 9 (profiles/short_qgram_r01.txt).  The text's alphabet is unknown here; the pattern's is the proxy.
-        bool seen[256] = {false};
-        int distinct = 0;
-        for (int i = 0; i < m && i < 16; ++i)
-            if (!seen[pat[i]]) { seen[pat[i]] = true; ++distinct; }
-        const int knob = env_int("BMX_QGRAM_UNIFORM", -1);   // measurement knob: 1 / 0 force one / four lengths
-        const bool uniform = knob >= 0 ? knob != 0 : !(m <= 9 && distinct <= 4);
-        if (uniform) {
+        if (filter == kQgram) {   // one length, m - 3 bytes (at most 8), for every residue
             for (int r = 0; r < 4; ++r) {
                 a->hmulr[r] = a->hmul;
                 a->f[r] = le_word(pat + r, 4) + a->hmul * le_word(pat + r + 4, std::min(m - 3, 8) - 4);
             }
         }
-    } else if (variant == BMX_VARIANT_WINDOW) {
+    } else if (filter_variant(filter) == BMX_VARIANT_WINDOW) {
         for (int k = 0; k < 5; ++k) a->bcast[k] = (uint32_t)pat[std::min(k, m - 1)] * 0x01010101u;
         const int q = std::min(m, 4);
-        a->mulc = q >= 4 ? 1u : (1u << (32 - 8 * q));
-        a->f[0] = le_word(pat, q) * a->mulc;
+        a->f[0] = le_word(pat, q) * (q >= 4 ? 1u : (1u << (32 - 8 * q)));   // 2^(32-8q) drops the bytes beyond q
     }
 }
 
-// FULL8: WINDOW compares whole 4-byte windows (m >= 4); QGRAM hashes all residues with one multiplier.
-// The kernels' FLAG parameter: QGRAM 1 = one multiplier for all residues; WINDOW 1 = whole 4-byte windows (m >= 4),
-// 2 / 3 / 4 = m of 1 / 2 / 3 bytes, 6 = five bytes at once (m = 5, 6 on small alphabets); everything else 1.
-static int uses_full8(int variant, const ScanArgs &a)
+// The scan_kernel instances of one filter kind: [tile is 32 KiB][positions mode].
+struct KernelRow {
+    const void *k[2][2];
+};
+template <Filter F>
+static KernelRow kernels_of()
 {
-    if (variant == BMX_VARIANT_WINDOW) return a.m >= 4 ? (a.window5 ? 6 : 1) : a.m + 1;
-    if (variant == BMX_VARIANT_QGRAM)
-        return (a.hmulr[0] == a.hmulr[3] && a.hmulr[1] == a.hmulr[3] && a.hmulr[2] == a.hmulr[3]) ? 1 : 0;
-    return 1;
+    return {{{(const void *)&scan_kernel<F, 16384, false>, (const void *)&scan_kernel<F, 16384, true>},
+             {(const void *)&scan_kernel<F, 32768, false>, (const void *)&scan_kernel<F, 32768, true>}}};
 }
-
-template <int VARIANT, int FULL8, int TILE, bool POSITIONS>
-static const void *kernel_ptr()
+static const void *scan_kernel_for(Filter filter, int tile, bool positions)
 {
-    return reinterpret_cast<const void *>(&scan_kernel<VARIANT, FULL8, TILE, POSITIONS>);
-}
-
-template <int TILE>
-static const void *pick_kernel_tile(int variant, int full8, bool positions)
-{
-    if (variant == BMX_VARIANT_QGRAM) {
-        if (full8) return positions ? kernel_ptr<kQgram, 1, TILE, true>() : kernel_ptr<kQgram, 1, TILE, false>();
-        return positions ? kernel_ptr<kQgram, 0, TILE, true>() : kernel_ptr<kQgram, 0, TILE, false>();
-    }
-    if (variant == BMX_VARIANT_WINDOW) {
-        switch (full8) {
-        case 2: return positions ? kernel_ptr<kWindow, 2, TILE, true>() : kernel_ptr<kWindow, 2, TILE, false>();
-        case 3: return positions ? kernel_ptr<kWindow, 3, TILE, true>() : kernel_ptr<kWindow, 3, TILE, false>();
-        case 4: return positions ? kernel_ptr<kWindow, 4, TILE, true>() : kernel_ptr<kWindow, 4, TILE, false>();
-        case 6: return positions ? kernel_ptr<kWindow, 6, TILE, true>() : kernel_ptr<kWindow, 6, TILE, false>();
-        default: return positions ? kernel_ptr<kWindow, 1, TILE, true>() : kernel_ptr<kWindow, 1, TILE, false>();
-        }
-    }
-    if (variant == BMX_VARIANT_MULTI_INTERNAL) return positions ? kernel_ptr<kMulti, 1, TILE, true>() : kernel_ptr<kMulti, 1, TILE, false>();
-    return positions ? kernel_ptr<kShiftAnd, 1, TILE, true>() : kernel_ptr<kShiftAnd, 1, TILE, false>();
-}
-
-static const void *pick_kernel(int variant, int full8, int tile, bool positions)
-{
-    switch (tile) {
-    case 16384: return pick_kernel_tile<16384>(variant, full8, positions);
-    case 32768: return pick_kernel_tile<32768>(variant, full8, positions);
-    default: return nullptr;
-    }
+    static const KernelRow rows[] = {kernels_of<kQgramPerResidue>(), kernels_of<kQgram>(), kernels_of<kWindow4>(),
+                                     kernels_of<kBytes1>(),          kernels_of<kBytes2>(), kernels_of<kBytes3>(),
+                                     kernels_of<kBytes5>(),          kernels_of<kShiftAnd>(), kernels_of<kMulti>()};
+    static_assert(sizeof rows / sizeof rows[0] == kFilterCount, "one row per filter kind, in the order of enum Filter");
+    return rows[filter].k[tile == 32768][positions];
 }
 
 // Device attributes (and the expand kernel's occupancy) are queried once per device, under a mutex: a search on
@@ -1561,12 +1505,12 @@ static int device_info(int device, int *sm_count, int *smem_optin, int *smem_sm,
     return BMX_OK;
 }
 
-int plan_scan(int device, int variant, int32_t m, bool positions, ScanArgs *a, ScanLaunch *out)
+int plan_scan(int device, Filter filter, int32_t m, bool positions, ScanArgs *a, ScanLaunch *out)
 {
     int sm_count = 0, smem_optin = 0, smem_sm = 0;
     if (int rc = device_info(device, &sm_count, &smem_optin, &smem_sm, nullptr)) return rc;
 
-    const bool multi = variant == BMX_VARIANT_MULTI_INTERNAL;
+    const bool multi = filter == kMulti;
     // profiles/tune_knobs.py: 32 KiB tiles, 2 CTAs/SM, 3 stages.  The multi-pattern variant keeps 37 KiB of tables in
     // shared memory: 16 KiB tiles leave room for a 4-stage ring next to them.
     int tile = multi ? env_int("BMX_MULTI_TILE", 16384) : env_int("BMX_TILE", 32768);
@@ -1594,33 +1538,25 @@ int plan_scan(int device, int variant, int32_t m, bool positions, ScanArgs *a, S
     if (stages < 2) return fail(BMX_E_NOMEM, "pattern of %d bytes leaves room for %d pipeline stages", m, stages);
     a->stages = (uint32_t)stages;
 
-    out->variant = variant;
+    out->filter = filter;
     out->tile_bytes = tile;
     out->smem_bytes = kCtlBytes + a->multi_smem + (size_t)stages * a->stage_stride;
     const int64_t tiles = (a->vlen + tile - 1) / tile;
     a->num_tiles = (uint32_t)tiles;
     a->num_segs = (uint32_t)(tiles * (tile / kSegBytes));
     a->num_blocks = (a->num_segs + kBlockSegs - 1) / kBlockSegs;
-    a->owner_offset = (variant == BMX_VARIANT_QGRAM || multi) ? -3 : 0;
+    a->owner_offset = filter_owner_offset(filter);
     a->coop_verify = env_int("BMX_COOP_VERIFY", 1) != 0 ? 1u : 0u;   // measurement knob
-    // WINDOW on m = 5, 6: the 4-byte window passes 1 in 256 positions of a 4-letter text and the scan becomes
-    // verification-bound (DNA: 2.0 / 2.2 TB/s).  The byte-parallel construction of the m <= 3 kernels, extended to five
-    // bytes (11 instructions per word instead of 7, exact for m = 5), is chosen when the pattern has <= 4 distinct
-    // bytes -- the same proxy for the text's alphabet as in the q-gram layout choice.  BMX_WINDOW5=0/1 forces either.
-    a->window5 = (variant == BMX_VARIANT_WINDOW && (m == 5 || m == 6) && env_int("BMX_WINDOW5", a->pat_distinct <= 4 ? 1 : 0) != 0) ? 1u : 0u;
     // Patterns whose flagged chunks are checked by the whole warp never gain from the dense path (profiles/verify_ab_r02.txt:
     // equal or faster at every density measured): 33 lanes = never.
-    const bool verifies = !(variant == BMX_VARIANT_SHIFTAND || (variant == BMX_VARIANT_WINDOW && (m <= 4 || (a->window5 && m == 5))));
-    const bool coop = verifies && a->coop_verify && a->pat_smem && a->verify_smem;
+    const bool coop = !filter_exact(filter, m) && a->coop_verify && a->pat_smem && a->verify_smem;
     a->dense_lanes = (uint32_t)std::max(1, std::min(33, env_int("BMX_DENSE_LANES", coop ? 33 : (int)(m >= 16 ? kDenseLanesLong : kDenseLanesShort))));
     // BMX_SPARE_SMS leaves SMs free for concurrently running kernels (the NCCL collectives of a
     // multi-GPU pipeline cannot start while a persistent grid holds every SM)
     const int spare = std::max(0, std::min(sm_count - 1, env_int("BMX_SPARE_SMS", 0)));
     out->grid = (int)std::min<int64_t>(tiles, (int64_t)(sm_count - spare) * ctas_per_sm);
 
-    const int full8 = uses_full8(variant, *a);
-    const void *k = pick_kernel(variant, full8, tile, positions);
-    if (!k) return fail(BMX_E_BADARG, "no kernel for variant %d tile %d", variant, tile);
+    const void *k = scan_kernel_for(filter, tile, positions);
     {
         // the opt-in shared-memory limit of a kernel is raised once per (device, kernel, size)
         static std::map<std::pair<int, const void *>, size_t> granted;
@@ -1638,8 +1574,7 @@ int plan_scan(int device, int variant, int32_t m, bool positions, ScanArgs *a, S
 
 int launch_scan(const ScanArgs &a, const ScanLaunch &l, bool positions, void *stream)
 {
-    const int full8 = uses_full8(l.variant, a);
-    const void *k = pick_kernel(l.variant, full8, l.tile_bytes, positions);
+    const void *k = scan_kernel_for(l.filter, l.tile_bytes, positions);
     void *params[] = {const_cast<ScanArgs *>(&a)};
     const cudaError_t e = cudaLaunchKernel(k, dim3((unsigned)l.grid), dim3(kThreads), params, l.smem_bytes,
                                            static_cast<cudaStream_t>(stream));
@@ -1688,18 +1623,6 @@ int launch_synth_fill(void *d_text, int64_t offset, int64_t len, uint64_t seed, 
                                                                              len, seed, alpha, sigma);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(BMX_E_CUDA, "synth_fill launch: %s", cudaGetErrorString(e));
-    return BMX_OK;
-}
-
-int launch_partition_count(const int64_t *d_pos, const unsigned long long *d_count, int64_t pos_cap,
-                           const int32_t *d_se, int32_t *d_ans, int32_t m, int32_t nparts, void *stream)
-{
-    if (nparts <= 0) return BMX_OK;
-    const int block = 128;
-    partition_count_kernel<<<(nparts + block - 1) / block, block, 0, static_cast<cudaStream_t>(stream)>>>(
-        d_pos, d_count, pos_cap, d_se, d_ans, m, nparts);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(BMX_E_CUDA, "partition_count launch: %s", cudaGetErrorString(e));
     return BMX_OK;
 }
 

@@ -13,9 +13,7 @@ struct bmx_scanner {
     // per-pattern state
     int32_t m = 0;             // pattern length (multi-pattern mode: the shortest one -- it bounds the start positions of a scan)
     int32_t m_halo = 0;        // multi-pattern mode: the longest pattern (sizes the staged halo); 0 = m
-    int variant = 0;
-    int requested_variant = -1;   // variant argument of the set_pattern call that built the block below (-1: nothing cached)
-    int qgram_knob = -1;          // BMX_QGRAM_UNIFORM at that time (a measurement knob that changes the filter constants)
+    bmx::Filter filter = bmx::kQgram;   // the scan kernel's filter kind (kMulti in multi-pattern mode)
     cudaEvent_t ev_pat = nullptr; // recorded behind the upload of the block
     cudaStream_t pat_stream = nullptr;
     std::vector<unsigned char> pat;

@@ -28,10 +28,12 @@ for line in out.splitlines():
     if m and name:
         kernels[name][m.group(1)] += 1
 
-want = sys.argv[1:] or ["scan_kernelILi1ELb1ELi32768ELb1E", "scan_kernelILi1ELb1ELi32768ELb0E", "scan_kernelILi2ELb1ELi32768ELb1E",
-                        "scan_kernelILi4ELb1ELi16384ELb1E", "expand_kernel", "xchg_post_kernel", "xchg_collect_kernel", "multi_split_kernel"]
+want = sys.argv[1:] or ["scan_kernelILNS_6FilterE1ELi32768ELb1E", "scan_kernelILNS_6FilterE1ELi32768ELb0E",
+                        "scan_kernelILNS_6FilterE2ELi32768ELb1E", "scan_kernelILNS_6FilterE8ELi16384ELb1E", "expand_kernel",
+                        "xchg_post_kernel", "xchg_collect_kernel", "multi_split_kernel"]
 print(f"# cuobjdump -sass {so.name}: instruction counts per kernel (static), grouped by opcode family")
-print("# scan_kernel<VARIANT, FULL8, TILE, POSITIONS>: Li1 = QGRAM, Li2 = WINDOW, Li4 = multi-pattern; Lb1/Lb0 = true/false")
+print("# scan_kernel<Filter, TILE, POSITIONS> (enum Filter, csrc/bmx_internal.h): FilterE1 = kQgram, FilterE2 = kWindow4, "
+      "FilterE8 = kMulti; Lb1/Lb0 = positions / count-only")
 for k, c in kernels.items():
     if not any(w in k for w in want):
         continue

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Measures every scan variant per (alphabet, pattern length) on one B200 and writes
-profiles/variants_<tag>.json -- the table that justifies bmx::resolve_variant()'s thresholds
+profiles/variants_<tag>.json -- the table that justifies the variant thresholds of bmx::choose_filter()
 (north star: "chosen per pattern length and justified by measurement").
 
     python profiles/sweep_variants.py --tag r01 [--gib 1] [--steps 10]

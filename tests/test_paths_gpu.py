@@ -1,7 +1,8 @@
 """GPU: every kernel instance and knob-selected branch driven on purpose, with the KMP matcher
 (oracle_kmp_search, no Boyer-Moore logic) as the truth.  Each case checks the full position list, capped lists
 (half the count and one entry), count-only mode and find_first_device, on an aligned and an odd-offset copy of
-the text.  The knobs are environment variables that plan_scan reads on every scan."""
+the text.  The knobs are environment variables: BMX_QGRAM_UNIFORM and BMX_WINDOW5 are read when the pattern is set
+(choose_filter), the others by plan_scan on every scan."""
 from __future__ import annotations
 
 import random
@@ -71,7 +72,7 @@ INSTANCES = [
 
 
 def verifies(variant: str, m: int, knobs: dict) -> bool:
-    """Whether the instance checks its candidates (the same rule as plan_scan)."""
+    """Whether the instance checks its candidates (the same rule as filter_exact)."""
     if variant == "shiftand" or (variant == "window" and m <= 4):
         return False
     return not (variant == "window" and m == 5 and knobs.get("BMX_WINDOW5") == 1)

@@ -129,6 +129,11 @@ class PendingExchange:
         """Waits for the collectives (the step's single host sync) and assembles the list on dst.
         Returns (total_count, per_rank_counts, positions_on_dst_or_None).
 
+        The list on dst is a prefix of the global ascending list, as the library exchange delivers it: whole
+        lists in rank order up to and including the first rank that holds fewer positions than its count.
+        Every rank knows every (count, held) pair from the gathered header, so every rank computes the same
+        cut; ranks behind it send no tail and dst posts no receive for them.
+
         On CUDA everything here runs on a side stream that depends only on the collectives, so a
         caller that has already queued later scans on its compute stream is not held up by them."""
         import contextlib
@@ -155,30 +160,34 @@ class PendingExchange:
             held_host = [int(header[2 * r + 1]) for r in range(world)]
             total_host = sum(counts_host)                              # every rank holds every count
             fast_cap, pos = self.fast_cap, self.positions_local
+            take, complete = [], True                                  # the same cut on every rank
+            for c, h in zip(counts_host, held_host):
+                take.append(min(c, h) if complete else 0)
+                complete = complete and h >= c
 
             gathered = None
             if rank == self.dst:
-                heads = [table[r, 2: 2 + min(held_host[r], fast_cap)] for r in range(world)]
-                if all(h <= fast_cap for h in held_host):
+                heads = [table[r, 2: 2 + min(take[r], fast_cap)] for r in range(world)]
+                if all(t <= fast_cap for t in take):
                     gathered = torch.cat(heads) if heads else torch.empty(0, dtype=torch.int64, device=self.device)
                 else:
-                    gathered = torch.empty(sum(held_host), dtype=torch.int64, device=self.device)
+                    gathered = torch.empty(sum(take), dtype=torch.int64, device=self.device)
                     off, reqs = 0, []
                     for r in range(world):
-                        k = min(held_host[r], fast_cap)
+                        k = min(take[r], fast_cap)
                         if k:
                             gathered[off: off + k] = heads[r]
-                        rest = held_host[r] - k
+                        rest = take[r] - k
                         if rest > 0:
                             if r == self.dst:
                                 gathered[off + k: off + k + rest] = pos[k: k + rest]
                             else:
                                 reqs.append(dist.irecv(gathered[off + k: off + k + rest], src=r, group=self.group))
-                        off += held_host[r]
+                        off += take[r]
                     for q in reqs:
                         q.wait()
-            elif held_host[rank] > fast_cap:
-                dist.send(pos[fast_cap:held_host[rank]].contiguous(), dst=self.dst, group=self.group)
+            elif take[rank] > fast_cap:
+                dist.send(pos[fast_cap:take[rank]].contiguous(), dst=self.dst, group=self.group)
         if cuda:
             torch.cuda.current_stream(self.device).wait_stream(side)   # later users of `gathered` are ordered after it
         return total_host, counts_host, gathered
@@ -214,6 +223,8 @@ def combine_hits_start(count_local, positions_local, *, group=None, device=None,
     count is the sum of the gathered counts: no separate all-reduce).  PendingExchange.finish() awaits it
     with a single host synchronisation; lists longer than fast_cap (dense texts) send their remainder to
     `dst` point-to-point.  Rank-order concatenation on `dst` is globally ascending: nothing is sorted.
+    The list on `dst` is a prefix of the global list, the same one the library exchange returns: it stops
+    behind the first rank whose list holds fewer positions than its count.
     """
     import torch
     import torch.distributed as dist
@@ -261,7 +272,9 @@ def sharded_search(shard_text, lo: int, pattern: bytes, *, max_positions: int, g
 
     shard_text holds the bytes [lo, end) of the global text (own range + halo, see
     shard_read_range).  Returns (total_count, per_rank_counts, positions_on_dst_or_None,
-    local_stats).  `local_scan(shard_text, pattern, pos_base, max_positions)` ->
+    local_stats).  The positions on dst are a prefix of the global ascending list: whole shard lists in
+    rank order, ending behind the first rank that found more than max_positions.
+    `local_scan(shard_text, pattern, pos_base, max_positions)` ->
     (count, positions_tensor, stats) defaults to the CUDA scan; the CPU tests inject a checker.
     """
     if local_scan is None:

@@ -47,6 +47,32 @@ int check_device(int device)
     return BMX_OK;
 }
 
+int check_text(const void *text, int64_t n, const char *who)
+{
+    if (n < 0 || (!text && n > 0)) return fail(BMX_E_BADARG, "%s: bad text (n=%lld)", who, (long long)n);
+    return BMX_OK;
+}
+
+int check_pattern(int32_t m)
+{
+    if (m <= 0 || m > BMX_MAX_PATTERN)
+        return fail(BMX_E_BADARG, "pattern length %d outside 1..%d (an empty pattern is rejected)", m, BMX_MAX_PATTERN);
+    return BMX_OK;
+}
+
+int check_pattern_set(int32_t npat, const char *const *pats, const int32_t *ms, int64_t *const *outs, const int64_t *caps,
+                      uint64_t *counts, const char *who)
+{
+    if (npat < 0 || (npat > 0 && (!pats || !ms || !counts))) return fail(BMX_E_BADARG, "%s: NULL argument or npat < 0", who);
+    for (int32_t k = 0; k < npat; ++k) {
+        if (!pats[k] || ms[k] <= 0 || ms[k] > BMX_MAX_PATTERN)
+            return fail(BMX_E_BADARG, "pattern %d: length %d outside 1..%d or NULL (an empty pattern is rejected)", k, ms[k], BMX_MAX_PATTERN);
+        if (outs && outs[k] && (!caps || caps[k] < 0)) return fail(BMX_E_BADARG, "pattern %d: pos_cap < 0 or missing", k);
+        counts[k] = 0;
+    }
+    return BMX_OK;
+}
+
 }  // namespace bmx
 
 using namespace bmx;
@@ -129,8 +155,7 @@ void bmx_scanner_destroy(bmx_scanner *s)
 int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t variant, void *stream)
 {
     if (!s || !pat) return fail(BMX_E_BADARG, "bmx_scanner_set_pattern: NULL argument");
-    if (m <= 0 || m > BMX_MAX_PATTERN)
-        return fail(BMX_E_BADARG, "pattern length %d outside 1..%d (an empty pattern is rejected)", m, BMX_MAX_PATTERN);
+    if (int rc = check_pattern(m)) return rc;
     if (variant < BMX_VARIANT_AUTO || variant > BMX_VARIANT_SHIFTAND)
         return fail(BMX_E_BADARG, "unknown variant %d", variant);
     BMX_CUDA(cudaSetDevice(s->device));
@@ -206,7 +231,7 @@ int bmx_scanner_begin(bmx_scanner *s, int64_t *d_pos_out, int64_t pos_cap, void 
 int bmx_scanner_scan(bmx_scanner *s, const void *d_text, int64_t n, int64_t pos_base, void *stream)
 {
     if (!s || s->m <= 0) return fail(BMX_E_BADARG, "bmx_scanner_scan: scanner has no pattern");
-    if (n < 0 || (!d_text && n > 0)) return fail(BMX_E_BADARG, "bmx_scanner_scan: bad text (n=%lld)", (long long)n);
+    if (int rc = check_text(d_text, n, "bmx_scanner_scan")) return rc;
     if (n < s->m) return BMX_OK;  // kernel1.cl:15,19: the loop is never entered
     BMX_CUDA(cudaSetDevice(s->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -347,24 +372,24 @@ namespace bmx {
 void ThreadCtx::release_buffers()
 {
     if (device < 0) return;
-    int keep = 0;
-    const bool have = cudaGetDevice(&keep) == cudaSuccess;
-    if (cudaSetDevice(device) == cudaSuccess) {
-        if (copy_stream) cudaStreamSynchronize(copy_stream);
-        if (scan_stream) cudaStreamSynchronize(scan_stream);
-        for (DevBuf *b : {&text, &pos, &misc, &aux}) {
-            if (b->p) cudaFree(b->p);
-            *b = DevBuf{};
+    {
+        ScopedDevice keep;
+        if (cudaSetDevice(device) == cudaSuccess) {
+            if (copy_stream) cudaStreamSynchronize(copy_stream);
+            if (scan_stream) cudaStreamSynchronize(scan_stream);
+            for (DevBuf *b : {&text, &pos, &misc, &aux}) {
+                if (b->p) cudaFree(b->p);
+                *b = DevBuf{};
+            }
+            for (int i = 0; i < kBounce; ++i) {
+                if (bounce[i]) cudaFreeHost(bounce[i]);
+                bounce[i] = nullptr;
+            }
+            bounce_bytes = 0;
+            if (h_small) cudaFreeHost(h_small);
+            h_small = nullptr;
         }
-        for (int i = 0; i < kBounce; ++i) {
-            if (bounce[i]) cudaFreeHost(bounce[i]);
-            bounce[i] = nullptr;
-        }
-        bounce_bytes = 0;
-        if (h_small) cudaFreeHost(h_small);
-        h_small = nullptr;
     }
-    if (have) cudaSetDevice(keep);
     (void)cudaGetLastError();
 }
 
@@ -373,16 +398,16 @@ ThreadCtx::~ThreadCtx()
     if (device < 0) return;
     // at process exit the CUDA runtime may already be gone: every call below then fails harmlessly
     release_buffers();
-    int keep = 0;
-    const bool have = cudaGetDevice(&keep) == cudaSuccess;
-    if (cudaSetDevice(device) == cudaSuccess) {
-        if (scanner) bmx_scanner_destroy(scanner);
-        if (copy_stream) cudaStreamDestroy(copy_stream);
-        if (scan_stream) cudaStreamDestroy(scan_stream);
-        for (cudaEvent_t e : events) cudaEventDestroy(e);
+    {
+        ScopedDevice keep;
+        if (cudaSetDevice(device) == cudaSuccess) {
+            if (scanner) bmx_scanner_destroy(scanner);
+            if (copy_stream) cudaStreamDestroy(copy_stream);
+            if (scan_stream) cudaStreamDestroy(scan_stream);
+            for (cudaEvent_t e : events) cudaEventDestroy(e);
+        }
+        scanner = nullptr;
     }
-    scanner = nullptr;
-    if (have) cudaSetDevice(keep);
     (void)cudaGetLastError();
 }
 
@@ -402,9 +427,16 @@ int get_ctx(int device, ThreadCtx **out)
     return BMX_OK;
 }
 
-int ensure_streams(ThreadCtx &c, int device, size_t nevents)
+int current_ctx(ThreadCtx **out)
 {
-    (void)device;
+    int device = 0;
+    if (int rc = check_device(0)) return rc;
+    BMX_CUDA(cudaGetDevice(&device));
+    return get_ctx(device, out);
+}
+
+int ensure_streams(ThreadCtx &c, size_t nevents)
+{
     if (!c.copy_stream) BMX_CUDA(cudaStreamCreateWithFlags(&c.copy_stream, cudaStreamNonBlocking));
     if (!c.scan_stream) BMX_CUDA(cudaStreamCreateWithFlags(&c.scan_stream, cudaStreamNonBlocking));
     while (c.events.size() < nevents) {
@@ -442,6 +474,16 @@ int scanner_begin_find(bmx_scanner *s, void *stream)
     return BMX_OK;
 }
 
+int search_once(bmx_scanner *s, const char *pat, int32_t m, int32_t variant, const void *d_text, int64_t n, int64_t pos_base,
+                int64_t *d_pos, int64_t pos_cap, uint64_t *count, bmx_stats *stats, void *stream)
+{
+    int rc = bmx_scanner_set_pattern(s, pat, m, variant, stream);
+    if (rc == BMX_OK) rc = bmx_scanner_begin(s, d_pos, pos_cap, stream);
+    if (rc == BMX_OK) rc = bmx_scanner_scan(s, d_text, n, pos_base, stream);
+    if (rc == BMX_OK) rc = bmx_scanner_finish(s, count, stats, stream);
+    return rc;
+}
+
 }  // namespace bmx
 
 extern "C" {
@@ -458,22 +500,13 @@ int bmx_search_device_ex(const void *d_text, int64_t n, const char *pat, int32_t
                          bmx_stats *stats, void *stream)
 {
     if (!count_out || !pat) return fail(BMX_E_BADARG, "bmx_search_device: pat/count_out must be non-NULL");
-    if (n < 0 || (!d_text && n > 0)) return fail(BMX_E_BADARG, "bmx_search_device: bad text (n=%lld)", (long long)n);
+    if (int rc = check_text(d_text, n, "bmx_search_device")) return rc;
     if (pos_cap < 0) return fail(BMX_E_BADARG, "pos_cap < 0");
-    int device = 0;
-    if (int rc = check_device(0)) return rc;
-    BMX_CUDA(cudaGetDevice(&device));
     ThreadCtx *c = nullptr;
-    if (int rc = get_ctx(device, &c)) return rc;
+    if (int rc = current_ctx(&c)) return rc;
     // CUDA events between the kernels cost microseconds per call: only a caller that asks for the times pays
-    const int keep_timing = c->scanner->timing_level;
-    c->scanner->timing_level = stats ? 2 : 0;
-    int rc = bmx_scanner_set_pattern(c->scanner, pat, m, variant, stream);
-    if (rc == BMX_OK) rc = bmx_scanner_begin(c->scanner, d_pos_out, pos_cap, stream);
-    if (rc == BMX_OK) rc = bmx_scanner_scan(c->scanner, d_text, n, pos_base, stream);
-    if (rc == BMX_OK) rc = bmx_scanner_finish(c->scanner, count_out, stats, stream);
-    c->scanner->timing_level = keep_timing;
-    return rc;
+    ScopedTiming timing(c->scanner, stats ? 2 : 0);
+    return search_once(c->scanner, pat, m, variant, d_text, n, pos_base, d_pos_out, pos_cap, count_out, stats, stream);
 }
 
 int bmx_search_device(const void *d_text, int64_t n, const char *pat, int32_t m, int64_t *d_pos_out,
@@ -495,24 +528,19 @@ int bmx_search_device(const void *d_text, int64_t n, const char *pat, int32_t m,
 int bmx_find_first_device(const void *d_text, int64_t n, const char *pat, int32_t m, int64_t *first_out, void *stream)
 {
     if (!first_out || !pat) return fail(BMX_E_BADARG, "bmx_find_first_device: pat/first_out must be non-NULL");
-    if (n < 0 || (!d_text && n > 0)) return fail(BMX_E_BADARG, "bmx_find_first_device: bad text (n=%lld)", (long long)n);
+    if (int rc = check_text(d_text, n, "bmx_find_first_device")) return rc;
     *first_out = -1;
-    int device = 0;
-    if (int rc = check_device(0)) return rc;
-    BMX_CUDA(cudaGetDevice(&device));
     ThreadCtx *c = nullptr;
-    if (int rc = get_ctx(device, &c)) return rc;
+    if (int rc = current_ctx(&c)) return rc;
     bmx_scanner *s = c->scanner;
     if (int rc = bmx_scanner_set_pattern(s, pat, m, BMX_VARIANT_AUTO, stream)) return rc;
     if (n < m) return BMX_OK;
     if ((uint64_t)n > kFindMask) return fail(BMX_E_BADARG, "bmx_find_first_device: texts beyond 2^47 bytes are not supported");
-    const int keep_timing = s->timing_level;
-    s->timing_level = 0;
+    ScopedTiming timing(s, 0);
     int rc = scanner_begin_find(s, stream);
     if (rc == BMX_OK) rc = bmx_scanner_scan(s, d_text, n, 0, stream);
     uint64_t partial = 0;
     if (rc == BMX_OK) rc = bmx_scanner_finish(s, &partial, nullptr, stream);
-    s->timing_level = keep_timing;
     if (rc == BMX_OK) *first_out = (int64_t) static_cast<volatile unsigned long long *>(s->h_result)[1];
     return rc;
 }

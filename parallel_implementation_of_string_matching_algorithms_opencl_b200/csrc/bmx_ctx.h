@@ -9,6 +9,7 @@
 
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "bmx_internal.h"
@@ -51,16 +52,75 @@ struct ThreadCtx {
     void release_buffers();  // text / positions / bounce buffers only (bmx_release_memory)
 };
 
+// ---- argument checks shared by the entry points (bmx_abi.cu).  Each returns BMX_OK or the code of bmx::fail.
 int check_device(int device);
-int get_ctx(int device, ThreadCtx **out);                        // the calling thread's context for `device`
-int ensure_streams(ThreadCtx &c, int device, size_t nevents);
+int check_text(const void *text, int64_t n, const char *who);   // n >= 0, and a text pointer unless n == 0
+int check_pattern(int32_t m);                                    // 1 <= m <= BMX_MAX_PATTERN
+// npat >= 0 with pats / ms / counts; then every pattern non-NULL, 1 <= ms[k] <= BMX_MAX_PATTERN, a cap for every
+// output buffer; counts[k] is zeroed as the loop passes it.
+int check_pattern_set(int32_t npat, const char *const *pats, const int32_t *ms, int64_t *const *outs, const int64_t *caps,
+                      uint64_t *counts, const char *who);
+
+int get_ctx(int device, ThreadCtx **out);   // the calling thread's context for `device`
+int current_ctx(ThreadCtx **out);           // ... for the calling thread's current device
+int ensure_streams(ThreadCtx &c, size_t nevents);
 // Grows b to at least `bytes` (never shrinks).  The old block may still be in use by work enqueued on the
 // context's streams, so they are drained before it is freed.  NOMEM leaves b empty.
 int ensure_buf(ThreadCtx &c, DevBuf &b, size_t bytes);
 int scanner_begin_find(bmx_scanner *s, void *stream);   // find-first search: count-only kernels + early stop (bmx_abi.cu)
+// One whole search with the scanner: set_pattern, begin, one scan of d_text[0..n), finish (bmx_abi.cu).
+int search_once(bmx_scanner *s, const char *pat, int32_t m, int32_t variant, const void *d_text, int64_t n, int64_t pos_base,
+                int64_t *d_pos, int64_t pos_cap, uint64_t *count, bmx_stats *stats, void *stream);
+
+// The position buffer of a search follows its count (DESIGN §2): a first guess of one hit per 64 bytes, at least
+// 1 Mi entries, never more than the want_cap positions the caller can use ...
+inline int64_t first_pos_cap(int64_t n, int32_t m, int64_t want_cap)
+{
+    return std::max<int64_t>(0, std::min<int64_t>({want_cap, n - m + 1, std::max<int64_t>(int64_t(1) << 20, n / 64)}));
+}
+// ... or the room c.pos already holds, if that is more.
+inline int64_t first_pos_room(const ThreadCtx &c, int64_t n, int32_t m, int64_t want_cap)
+{
+    const int64_t cap = first_pos_cap(n, m, want_cap), owned = (int64_t)(c.pos.cap / 8);
+    return owned > cap ? std::min(want_cap, owned) : cap;
+}
+
+// One shard of a host text through the calling GPU's context (bmx_host.cu, used by bmx_multi.cu).
+int ingest_shard(ThreadCtx &ctx, int device, const char *text, int64_t n, const char *pat, int32_t m, int64_t pos_base,
+                 int64_t want_cap, uint64_t *count, int64_t *dev_cap);
+
 // K patterns in one pass over device-resident text (bmx_multipat.cu)
-bool multi_set_eligible(int32_t npat, const int32_t *ms);
+bool multi_eligible(int32_t npat, const int32_t *ms);
 int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, int32_t npat, const char *const *pats,
                         const int32_t *ms, int64_t *const *d_out, const int64_t *caps, uint64_t *counts, cudaStream_t st);
+
+// Sets the scanner's timing level (bmx_scanner_set_timing) for the scope and restores the caller's level after it.
+class ScopedTiming {
+public:
+    ScopedTiming(bmx_scanner *s, int level) : s_(s), keep_(s->timing_level) { s_->timing_level = level; }
+    ~ScopedTiming() { s_->timing_level = keep_; }
+    ScopedTiming(const ScopedTiming &) = delete;
+    ScopedTiming &operator=(const ScopedTiming &) = delete;
+
+private:
+    bmx_scanner *s_;
+    int keep_;
+};
+
+// Restores the calling thread's current device when the scope ends.
+class ScopedDevice {
+public:
+    ScopedDevice() : have_(cudaGetDevice(&keep_) == cudaSuccess) {}
+    ~ScopedDevice()
+    {
+        if (have_) cudaSetDevice(keep_);
+    }
+    ScopedDevice(const ScopedDevice &) = delete;
+    ScopedDevice &operator=(const ScopedDevice &) = delete;
+
+private:
+    int keep_ = 0;
+    bool have_;
+};
 
 }  // namespace bmx

@@ -31,8 +31,7 @@
 #include <cstring>
 #include <new>
 
-#include "bmx_internal.h"
-#include "bmx_scanner.h"
+#include "bmx_ctx.h"
 
 namespace bmx {
 
@@ -267,14 +266,6 @@ struct bmx_exchange {
     unsigned long long timeout_ns = 20ull * 1000 * 1000 * 1000;
 };
 
-#define BMX_CUDA(call)                                                                                   \
-    do {                                                                                                 \
-        cudaError_t e_ = (call);                                                                         \
-        if (e_ != cudaSuccess)                                                                           \
-            return fail(e_ == cudaErrorMemoryAllocation ? BMX_E_NOMEM : BMX_E_CUDA, "%s: %s", #call,     \
-                        cudaGetErrorString(e_));                                                         \
-    } while (0)
-
 static XArgs make_args(const bmx_exchange *x, uint64_t seq)
 {
     XArgs a{};
@@ -307,12 +298,7 @@ int bmx_exchange_create(int device, int rank, int world, int dst, int64_t head_c
         return fail(BMX_E_BADARG, "bmx_exchange_create: rank %d / dst %d / world %d (1..%d)", rank, dst, world, kMaxRanks);
     if (head_cap < 0 || tail_cap < 0 || depth < 2 || depth > 64)
         return fail(BMX_E_BADARG, "bmx_exchange_create: head_cap/tail_cap >= 0 and 2 <= depth <= 64 required");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        (void)cudaGetLastError();
-        return fail(BMX_E_NODEVICE, "no CUDA device visible; libbmx has no CPU path");
-    }
-    if (device < 0 || device >= ndev) return fail(BMX_E_BADARG, "device %d out of range (0..%d)", device, ndev - 1);
+    if (int rc = check_device(device)) return rc;
     BMX_CUDA(cudaSetDevice(device));
     bmx_exchange *x = new (std::nothrow) bmx_exchange();
     if (!x) return fail(BMX_E_NOMEM, "out of host memory");
@@ -323,10 +309,7 @@ int bmx_exchange_create(int device, int rank, int world, int dst, int64_t head_c
     x->depth = depth;
     x->head_cap = head_cap;
     x->tail_cap = tail_cap;
-    if (const char *e = getenv("BMX_XCHG_TIMEOUT_MS")) {
-        const long ms = atol(e);
-        if (ms > 0) x->timeout_ns = (unsigned long long)ms * 1000000ull;
-    }
+    if (const int ms = env_int("BMX_XCHG_TIMEOUT_MS", 0); ms > 0) x->timeout_ns = (unsigned long long)ms * 1000000ull;
     // the same offsets on every rank (a writer computes addresses inside dst's mailbox from them); only dst
     // backs the list areas with memory
     auto align = [](size_t v) { return (v + 255) & ~size_t(255); };
@@ -407,30 +390,23 @@ int bmx_exchange_connect_local(bmx_exchange *const *all, int world)
     for (int r = 0; r < world; ++r)
         if (!all[r] || all[r]->world != world || all[r]->rank != r)
             return fail(BMX_E_BADARG, "bmx_exchange_connect_local: entry %d is not rank %d of a world of %d", r, r, world);
-    int keep = 0;
-    cudaGetDevice(&keep);
+    ScopedDevice keep;
     for (int a = 0; a < world; ++a) {
         BMX_CUDA(cudaSetDevice(all[a]->device));
         for (int b = 0; b < world; ++b) {
             if (all[b]->device != all[a]->device) {
                 int can = 0;
                 BMX_CUDA(cudaDeviceCanAccessPeer(&can, all[a]->device, all[b]->device));
-                if (!can) {
-                    cudaSetDevice(keep);
-                    return fail(BMX_E_EXCHANGE, "device %d cannot access device %d", all[a]->device, all[b]->device);
-                }
+                if (!can) return fail(BMX_E_EXCHANGE, "device %d cannot access device %d", all[a]->device, all[b]->device);
                 const cudaError_t e = cudaDeviceEnablePeerAccess(all[b]->device, 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) {
-                    cudaSetDevice(keep);
+                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled)
                     return fail(BMX_E_EXCHANGE, "cudaDeviceEnablePeerAccess(%d -> %d): %s", all[a]->device, all[b]->device, cudaGetErrorString(e));
-                }
                 (void)cudaGetLastError();
             }
             all[a]->peer[b] = all[b]->mailbox;
         }
         all[a]->connected = true;
     }
-    cudaSetDevice(keep);
     return BMX_OK;
 }
 

@@ -60,34 +60,19 @@ bool is_pinned_host(const void *p)
     return attr.type == cudaMemoryTypeHost;
 }
 
-long env_long(const char *name, long fallback)
-{
-    const char *e = getenv(name);
-    return (e && *e) ? atol(e) : fallback;
-}
-
-// First guess for the position buffer of a text of n bytes (entries): one hit per 64 bytes, at least 1 Mi.
-int64_t first_pos_cap(int64_t n, int32_t m, int64_t want_cap)
-{
-    return std::max<int64_t>(0, std::min<int64_t>({want_cap, n - m + 1, std::max<int64_t>(int64_t(1) << 20, n / 64)}));
-}
-
 // One search over device-resident text with a position buffer that follows the count: first pass with the
 // cached buffer, and only if the text holds more hits than it has room for (and the caller wants them) a
 // second pass with a buffer of the right size.  On return ctx.pos holds min(count, *dev_cap) positions.
 int scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, const char *pat, int32_t m, int32_t variant,
                   int64_t pos_base, int64_t want_cap, uint64_t *count, int64_t *dev_cap, bmx_stats *stats)
 {
-    int64_t cap = first_pos_cap(n, m, want_cap);
-    if ((int64_t)(c.pos.cap / 8) > cap) cap = std::min<int64_t>(want_cap, (int64_t)(c.pos.cap / 8));  // room we already own
+    int64_t cap = first_pos_room(c, n, m, want_cap);
     for (int pass = 0; pass < 2; ++pass) {
         if (cap > 0)
             if (int rc = ensure_buf(c, c.pos, (size_t)cap * 8)) return rc;
-        int rc = bmx_scanner_set_pattern(c.scanner, pat, m, variant, c.scan_stream);
-        if (rc == BMX_OK) rc = bmx_scanner_begin(c.scanner, cap > 0 ? static_cast<int64_t *>(c.pos.p) : nullptr, cap, c.scan_stream);
-        if (rc == BMX_OK) rc = bmx_scanner_scan(c.scanner, d_text, n, pos_base, c.scan_stream);
-        if (rc == BMX_OK) rc = bmx_scanner_finish(c.scanner, count, stats, c.scan_stream);
-        if (rc != BMX_OK) return rc;
+        if (int rc = search_once(c.scanner, pat, m, variant, d_text, n, pos_base, cap > 0 ? static_cast<int64_t *>(c.pos.p) : nullptr,
+                                 cap, count, stats, c.scan_stream))
+            return rc;
         const int64_t need = std::min<int64_t>(want_cap, (int64_t)*count);
         if (need <= cap) break;
         cap = need;
@@ -102,13 +87,12 @@ int scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, const ch
 // landing area right behind the kernels, so that the call synchronises once instead of twice (count, then positions).
 // Falls back to the resident re-scan when the text holds more hits than the position buffer (scan_resident).
 constexpr int64_t kSmallHostBytes = int64_t(4) << 20;
-int small_host_search(ThreadCtx &c, int device, const char *text, int64_t n, const char *pat, int32_t m, int32_t variant,
+int small_host_search(ThreadCtx &c, const char *text, int64_t n, const char *pat, int32_t m, int32_t variant,
                       int64_t *pos_out, int64_t want_cap, uint64_t *count_out, bmx_stats *stats)
 {
-    if (int rc = ensure_streams(c, device, 0)) return rc;
+    if (int rc = ensure_streams(c, 0)) return rc;
     if (int rc = ensure_buf(c, c.text, (size_t)n + 16)) return rc;
-    int64_t cap = first_pos_cap(n, m, want_cap);
-    if ((int64_t)(c.pos.cap / 8) > cap) cap = std::min<int64_t>(want_cap, (int64_t)(c.pos.cap / 8));
+    const int64_t cap = first_pos_room(c, n, m, want_cap);
     if (cap > 0)
         if (int rc = ensure_buf(c, c.pos, (size_t)cap * 8)) return rc;
     if (cap > 0 && !c.h_small) BMX_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&c.h_small), (size_t)kSmallSpec * 8, cudaHostAllocDefault));
@@ -148,8 +132,8 @@ struct Ingest {
     // in
     int64_t want_cap = 0;        // positions the caller can use (0: count only)
     bool find_first = false;     // stop copying and scanning behind the first match
-    bool need_resident = false;  // the caller wants to re-scan the device copy (bmx_search_multi)
-    bool copy_only = false;      // ingest without scanning (the caller scans the resident copy itself)
+    bool copy_only = false;      // ingest without scanning into the resident layout: the caller scans the device copy
+                                 // itself (bmx_search_multi); NOMEM when the text does not fit
     // out
     uint64_t count = 0;
     int64_t dev_cap = 0;         // ctx.pos holds min(count, dev_cap) positions
@@ -168,25 +152,24 @@ int ingest_and_scan(ThreadCtx &ctx, int device, const char *text, int64_t n, con
     io->first = -1;
     io->resident = false;
     io->stats = bmx_stats{};
-    if (n < m && !(io->need_resident && n > 0)) return BMX_OK;
-    if (io->copy_only && !io->need_resident) return fail(BMX_E_BADARG, "copy-only ingest needs the resident layout");
+    if (n < m && !(io->copy_only && n > 0)) return BMX_OK;
     BMX_CUDA(cudaSetDevice(device));
 
-    int64_t chunk = std::max<long>(1, env_long("BMX_H2D_CHUNK_MB", 64)) << 20;
-    if (const long kb = env_long("BMX_H2D_CHUNK_KB", 0)) chunk = (int64_t)kb << 10;   // test knob: many tiny chunks
+    int64_t chunk = (int64_t)std::max(1, env_int("BMX_H2D_CHUNK_MB", 64)) << 20;
+    if (const int kb = env_int("BMX_H2D_CHUNK_KB", 0)) chunk = (int64_t)kb << 10;   // test knob: many tiny chunks
     chunk = (std::max<int64_t>(chunk, (int64_t)m * 2) + 15) & ~int64_t(15);
     const int64_t nchunks = (n + chunk - 1) / chunk;
     // events: [0] copy of chunk k done, [1 .. kBounce] bounce buffer free, [1+kBounce .. +kRing) ring slot free,
     // then two "find-first result of scan q is in host memory" events.  An event is re-recorded freely: a stream
     // wait captures the record that precedes it.
     const size_t ev_copy = 0, ev_bounce = 1, ev_slot = 1 + kBounce, ev_find = 1 + kBounce + kRing;
-    if (int rc = ensure_streams(*c, device, ev_find + 2)) return rc;
+    if (int rc = ensure_streams(*c, ev_find + 2)) return rc;
     // work of an earlier call on these streams may still use the cached buffers
     const int64_t carry = m - 1;
     const size_t pre = ((size_t)carry + 15 + 16) & ~size_t(15);
 
     // ---- layout of the device copy
-    const long limit_mb = env_long("BMX_RESIDENT_MAX_MB", -1);
+    const int limit_mb = env_int("BMX_RESIDENT_MAX_MB", -1);
     const size_t resident_need = (size_t)n + 16;
     bool resident;
     if (limit_mb >= 0) {
@@ -201,7 +184,7 @@ int ingest_and_scan(ThreadCtx &ctx, int device, const char *text, int64_t n, con
     }
     if (resident && ensure_buf(*c, c->text, resident_need) != BMX_OK) resident = false;   // fragmentation etc.: stream it
     if (!resident) {
-        if (io->need_resident) return fail(BMX_E_NOMEM, "text of %lld bytes does not fit on the device", (long long)n);
+        if (io->copy_only) return fail(BMX_E_NOMEM, "text of %lld bytes does not fit on the device", (long long)n);
         const size_t slot_stride = pre + (size_t)chunk + 16;
         if (int rc = ensure_buf(*c, c->text, slot_stride * kRing)) return rc;
     }
@@ -210,7 +193,7 @@ int ingest_and_scan(ThreadCtx &ctx, int device, const char *text, int64_t n, con
     io->resident = resident;
 
     const bool pinned = is_pinned_host(text);
-    int staging_threads = (int)env_long("BMX_STAGING_THREADS", 16);  // host threads filling a bounce buffer: 8 -> 39.9, 16 -> 42.8, 32 -> 43.2 GB/s (profiles/e2e_host_memory_r02.txt)
+    int staging_threads = env_int("BMX_STAGING_THREADS", 16);  // host threads filling a bounce buffer: 8 -> 39.9, 16 -> 42.8, 32 -> 43.2 GB/s (profiles/e2e_host_memory_r02.txt)
     staging_threads = (int)std::max(1u, std::min<unsigned>((unsigned)std::max(1, std::min(64, staging_threads)), std::thread::hardware_concurrency()));
     if (!pinned && c->bounce_bytes < (size_t)std::min(chunk, n)) {
         for (int b = 0; b < kBounce; ++b) {
@@ -222,8 +205,7 @@ int ingest_and_scan(ThreadCtx &ctx, int device, const char *text, int64_t n, con
         c->bounce_bytes = (size_t)std::min(chunk, n);
     }
 
-    int64_t cap = io->find_first ? 0 : first_pos_cap(n, m, io->want_cap);
-    if (!io->find_first && (int64_t)(c->pos.cap / 8) > cap) cap = std::min<int64_t>(io->want_cap, (int64_t)(c->pos.cap / 8));
+    int64_t cap = io->find_first ? 0 : first_pos_room(*c, n, m, io->want_cap);
     for (int pass = 0; pass < 2; ++pass) {
         if (cap > 0)
             if (int rc = ensure_buf(*c, c->pos, (size_t)cap * 8)) return rc;
@@ -331,7 +313,6 @@ int ingest_and_scan(ThreadCtx &ctx, int device, const char *text, int64_t n, con
 }  // namespace
 
 namespace bmx {
-// used by bmx_multi.cu: one shard of a host text through the calling GPU's context
 int ingest_shard(ThreadCtx &ctx, int device, const char *text, int64_t n, const char *pat, int32_t m, int64_t pos_base,
                  int64_t want_cap, uint64_t *count, int64_t *dev_cap)
 {
@@ -350,10 +331,9 @@ int bmx_search_ex(int device, const char *text, int64_t n, const char *pat, int3
                   int64_t pos_cap, uint64_t *count_out, int32_t variant, bmx_stats *stats)
 {
     if (!count_out || !pat) return fail(BMX_E_BADARG, "bmx_search: pat/count_out must be non-NULL");
-    if (n < 0 || (!text && n > 0)) return fail(BMX_E_BADARG, "bmx_search: bad text (n=%lld)", (long long)n);
+    if (int rc = check_text(text, n, "bmx_search")) return rc;
     if (pos_cap < 0) return fail(BMX_E_BADARG, "pos_cap < 0");
-    if (m <= 0 || m > BMX_MAX_PATTERN)
-        return fail(BMX_E_BADARG, "pattern length %d outside 1..%d (an empty pattern is rejected)", m, BMX_MAX_PATTERN);
+    if (int rc = check_pattern(m)) return rc;
     ThreadCtx *c = nullptr;
     if (int rc = get_ctx(device, &c)) return rc;
     *count_out = 0;
@@ -361,14 +341,9 @@ int bmx_search_ex(int device, const char *text, int64_t n, const char *pat, int3
     if (n < m) return BMX_OK;
     // CUDA-event instrumentation only when the caller asks for the times: the records cost ~15 us per call
     // (profiles/call_latency_r02.txt), which is nothing for 4 GiB and a fifth of a call on the reference's 500 KB fixture
-    struct TimingGuard {
-        bmx_scanner *s;
-        int keep;
-        TimingGuard(bmx_scanner *sc, int level) : s(sc), keep(sc->timing_level) { s->timing_level = level; }
-        ~TimingGuard() { s->timing_level = keep; }
-    } timing_guard(c->scanner, stats ? 2 : 0);
-    if (n <= kSmallHostBytes && env_long("BMX_SMALL_HOST", 1) != 0 && env_long("BMX_RESIDENT_MAX_MB", -1) < 0 && env_long("BMX_H2D_CHUNK_KB", 0) == 0)
-        return small_host_search(*c, device, text, n, pat, m, variant, pos_out, pos_out ? std::min(pos_cap, n - m + 1) : 0, count_out, stats);
+    ScopedTiming timing(c->scanner, stats ? 2 : 0);
+    if (n <= kSmallHostBytes && env_int("BMX_SMALL_HOST", 1) != 0 && env_int("BMX_RESIDENT_MAX_MB", -1) < 0 && env_int("BMX_H2D_CHUNK_KB", 0) == 0)
+        return small_host_search(*c, text, n, pat, m, variant, pos_out, pos_out ? std::min(pos_cap, n - m + 1) : 0, count_out, stats);
     Ingest io;
     io.want_cap = pos_out ? std::min(pos_cap, n - m + 1) : 0;
     if (int rc = ingest_and_scan(*c, device, text, n, pat, m, 0, variant, &io)) return rc;
@@ -383,10 +358,9 @@ int bmx_search_ex(int device, const char *text, int64_t n, const char *pat, int3
 int bmx_search(const char *text, int64_t n, const char *pat, int32_t m, int64_t *pos_out, int64_t pos_cap,
                uint64_t *count_out)
 {
-    int device = 0;
-    if (int rc = check_device(0)) return rc;
-    BMX_CUDA(cudaGetDevice(&device));
-    return bmx_search_ex(device, text, n, pat, m, pos_out, pos_cap, count_out, BMX_VARIANT_AUTO, nullptr);
+    ThreadCtx *c = nullptr;
+    if (int rc = current_ctx(&c)) return rc;
+    return bmx_search_ex(c->device, text, n, pat, m, pos_out, pos_cap, count_out, BMX_VARIANT_AUTO, nullptr);
 }
 
 // K patterns over one host text: the text crosses PCIe ONCE (chunked, overlapped with the first scan); after
@@ -395,14 +369,8 @@ int bmx_search(const char *text, int64_t n, const char *pat, int32_t m, int64_t 
 int bmx_search_multi(int device, const char *text, int64_t n, int32_t npat, const char *const *pats, const int32_t *ms,
                      int64_t *const *pos_out, const int64_t *pos_cap, uint64_t *counts)
 {
-    if (npat < 0 || (npat > 0 && (!pats || !ms || !counts))) return fail(BMX_E_BADARG, "bmx_search_multi: NULL argument or npat < 0");
-    if (n < 0 || (!text && n > 0)) return fail(BMX_E_BADARG, "bmx_search_multi: bad text (n=%lld)", (long long)n);
-    for (int32_t k = 0; k < npat; ++k) {
-        if (!pats[k] || ms[k] <= 0 || ms[k] > BMX_MAX_PATTERN)
-            return fail(BMX_E_BADARG, "pattern %d: length %d outside 1..%d or NULL (an empty pattern is rejected)", k, ms[k], BMX_MAX_PATTERN);
-        if (pos_out && pos_out[k] && (!pos_cap || pos_cap[k] < 0)) return fail(BMX_E_BADARG, "pattern %d: pos_cap < 0 or missing", k);
-        counts[k] = 0;
-    }
+    if (int rc = check_text(text, n, "bmx_search_multi")) return rc;
+    if (int rc = check_pattern_set(npat, pats, ms, pos_out, pos_cap, counts, "bmx_search_multi")) return rc;
     ThreadCtx *c = nullptr;
     if (int rc = get_ctx(device, &c)) return rc;
     if (npat == 0 || n == 0) return BMX_OK;
@@ -419,7 +387,6 @@ int bmx_search_multi(int device, const char *text, int64_t n, int32_t npat, cons
     // the text crosses PCIe once; then all patterns in one pass over the resident copy when the set is eligible
     // (bmx_multipat.cu), else pattern by pattern
     Ingest io;
-    io.need_resident = true;
     io.copy_only = true;
     int32_t m_min = ms[0];
     for (int32_t k = 1; k < npat; ++k) m_min = std::min(m_min, ms[k]);
@@ -437,7 +404,7 @@ int bmx_search_multi(int device, const char *text, int64_t n, int32_t npat, cons
     }
     if (rc != BMX_OK) return rc;
     const unsigned char *d_text = static_cast<const unsigned char *>(c->text.p);
-    if (multi_set_eligible(npat, ms)) {
+    if (multi_eligible(npat, ms)) {
         // device-side output buffers: a first guess per pattern (one hit per 64 bytes), grown to the counts if a
         // pattern turns out denser -- the resident text is simply scanned again
         std::vector<int64_t> dev_cap((size_t)npat, 0);
@@ -486,20 +453,16 @@ int bmx_search_multi(int device, const char *text, int64_t n, int32_t npat, cons
 int bmx_find_first(const char *text, int64_t n, const char *pat, int32_t m, int64_t *first_out)
 {
     if (!first_out || !pat) return fail(BMX_E_BADARG, "bmx_find_first: pat/first_out must be non-NULL");
-    if (n < 0 || (!text && n > 0)) return fail(BMX_E_BADARG, "bmx_find_first: bad text (n=%lld)", (long long)n);
-    if (m <= 0 || m > BMX_MAX_PATTERN)
-        return fail(BMX_E_BADARG, "pattern length %d outside 1..%d (an empty pattern is rejected)", m, BMX_MAX_PATTERN);
+    if (int rc = check_text(text, n, "bmx_find_first")) return rc;
+    if (int rc = check_pattern(m)) return rc;
     *first_out = -1;
-    int device = 0;
-    if (int rc = check_device(0)) return rc;
-    BMX_CUDA(cudaGetDevice(&device));
     ThreadCtx *c = nullptr;
-    if (int rc = get_ctx(device, &c)) return rc;
+    if (int rc = current_ctx(&c)) return rc;
     if (n < m) return BMX_OK;
     if ((uint64_t)n > kFindMask) return fail(BMX_E_BADARG, "bmx_find_first: texts beyond 2^47 bytes are not supported");
     Ingest io;
     io.find_first = true;
-    if (int rc = ingest_and_scan(*c, device, text, n, pat, m, 0, BMX_VARIANT_AUTO, &io)) return rc;
+    if (int rc = ingest_and_scan(*c, c->device, text, n, pat, m, 0, BMX_VARIANT_AUTO, &io)) return rc;
     *first_out = io.first;
     return BMX_OK;
 }
@@ -509,8 +472,7 @@ int bmx_search_partitions(const char *text, const char *pat, const int32_t *se, 
 {
     if (!pat || !se || !ans || nparts < 0 || (!text && nparts > 0))
         return fail(BMX_E_BADARG, "bmx_search_partitions: NULL argument or nparts < 0");
-    if (m <= 0 || m > BMX_MAX_PATTERN)
-        return fail(BMX_E_BADARG, "pattern length %d outside 1..%d (an empty pattern is rejected)", m, BMX_MAX_PATTERN);
+    if (int rc = check_pattern(m)) return rc;
     if (nparts == 0) return BMX_OK;
 
     // The reference hands its own tables to the kernel (BoyreMoore.cpp:268-269).  The device scan
@@ -538,12 +500,9 @@ int bmx_search_partitions(const char *text, const char *pat, const int32_t *se, 
     const int64_t span = hi - lo + 1;
     if (span < m) return BMX_OK;
 
-    int device = 0;
-    if (int rc = check_device(0)) return rc;
-    BMX_CUDA(cudaGetDevice(&device));
     ThreadCtx *c = nullptr;
-    if (int rc = get_ctx(device, &c)) return rc;
-    if (int rc = ensure_streams(*c, device, 1)) return rc;
+    if (int rc = current_ctx(&c)) return rc;
+    if (int rc = ensure_streams(*c, 1)) return rc;
     cudaStream_t st = c->scan_stream;
     // One work-item of the reference = one count-only scan of its inclusive range (occurrences lying fully
     // inside it, kernel1.cl:15,19): no position list, so no memory proportional to the text beyond the text.
@@ -554,8 +513,7 @@ int bmx_search_partitions(const char *text, const char *pat, const int32_t *se, 
     BMX_CUDA(cudaMemsetAsync(d_counts, 0, (size_t)nparts * 8, st));
     BMX_CUDA(cudaMemcpyAsync(d_text, text + lo, (size_t)span, cudaMemcpyHostToDevice, st));
     if (int rc = bmx_scanner_set_pattern(c->scanner, pat, m, BMX_VARIANT_AUTO, st)) return rc;
-    const int keep_timing = c->scanner->timing_level;
-    c->scanner->timing_level = 0;
+    ScopedTiming timing(c->scanner, 0);
     int rc = BMX_OK;
     for (int32_t id = 0; id < nparts && rc == BMX_OK; ++id) {
         const int64_t a = se[2 * id], len = (int64_t)se[2 * id + 1] - a + 1;
@@ -565,7 +523,6 @@ int bmx_search_partitions(const char *text, const char *pat, const int32_t *se, 
         if (rc == BMX_OK && cudaMemcpyAsync(d_counts + id, result_slot(c->scanner), 8, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
             rc = fail(BMX_E_CUDA, "bmx_search_partitions: %s", cudaGetErrorString(cudaGetLastError()));
     }
-    c->scanner->timing_level = keep_timing;
     std::vector<unsigned long long> h_counts((size_t)nparts, 0);
     if (rc == BMX_OK && cudaMemcpyAsync(h_counts.data(), d_counts, (size_t)nparts * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
         rc = fail(BMX_E_CUDA, "bmx_search_partitions: %s", cudaGetErrorString(cudaGetLastError()));

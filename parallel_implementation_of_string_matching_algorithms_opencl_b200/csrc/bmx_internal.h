@@ -3,6 +3,7 @@
 
 #include <cstddef>
 #include <cstdint>
+#include <cstdlib>
 
 #include <vector_types.h>   // uint2 (CUDA toolkit header, plain C++)
 
@@ -175,5 +176,22 @@ constexpr uint32_t kMultiSlotMul = 0x85EBCA6Bu;
 constexpr uint32_t kHashMul2 = 0xC2B2AE3Du;
 constexpr size_t kMultiSmemBytes = (size_t)kMultiBitmapWords * 4 + (size_t)kMultiSlots * 8 + (size_t)kMultiMaxPatterns * 8;
 constexpr unsigned long long kFindMask = (1ull << 47) - 1;   // find-first keys: positions below 2^47
+
+// ---- host helpers -------------------------------------------------------------------------
+// The first min(nbytes, 4) bytes at p as a little-endian word (the q-gram hashes' view of the text).
+inline uint32_t le_word(const unsigned char *p, int nbytes)
+{
+    uint32_t w = 0;
+    for (int i = 0; i < nbytes && i < 4; ++i) w |= (uint32_t)p[i] << (8 * i);
+    return w;
+}
+// Hash multiplier of a word that contributes `bytes` bytes to a gram: K << (32 - 8*bytes) drops the bytes beyond it.
+inline uint32_t gram_multiplier(uint32_t K, int bytes) { return bytes >= 4 ? K : (bytes == 0 ? 0u : (K << (32 - 8 * bytes))); }
+// An integer environment knob, read on every call (tests change them between calls).
+inline int env_int(const char *name, int fallback)
+{
+    const char *v = getenv(name);
+    return (v && *v) ? atoi(v) : fallback;
+}
 
 }  // namespace bmx

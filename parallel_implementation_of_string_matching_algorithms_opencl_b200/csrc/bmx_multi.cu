@@ -17,11 +17,6 @@
 
 using namespace bmx;
 
-namespace bmx {
-int ingest_shard(ThreadCtx &ctx, int device, const char *text, int64_t n, const char *pat, int32_t m, int64_t pos_base,
-                 int64_t want_cap, uint64_t *count, int64_t *dev_cap);   // bmx_host.cu
-}
-
 extern "C" {
 
 struct bmx_mg {
@@ -97,8 +92,7 @@ int bmx_mg_create(int ngpus, bmx_mg **out)
     BMX_CUDA(cudaGetDeviceCount(&have));
     if (ngpus <= 0) ngpus = have;
     if (ngpus > have) return fail(BMX_E_BADARG, "bmx_mg_create: %d GPUs requested, %d visible", ngpus, have);
-    int keep = 0;
-    cudaGetDevice(&keep);
+    ScopedDevice keep;
     bmx_mg *mg = new (std::nothrow) bmx_mg();
     if (!mg) return fail(BMX_E_NOMEM, "out of host memory");
     for (int d = 0; d < ngpus; ++d) {
@@ -109,13 +103,11 @@ int bmx_mg_create(int ngpus, bmx_mg **out)
         if (rc != BMX_OK) {
             delete c;
             bmx_mg_destroy(mg);
-            cudaSetDevice(keep);
             return rc;
         }
         mg->devices.push_back(d);
         mg->ctx.push_back(c);
     }
-    cudaSetDevice(keep);
     *out = mg;
     return BMX_OK;
 }
@@ -123,11 +115,9 @@ int bmx_mg_create(int ngpus, bmx_mg **out)
 void bmx_mg_destroy(bmx_mg *mg)
 {
     if (!mg) return;
-    int keep = 0;
-    cudaGetDevice(&keep);
+    ScopedDevice keep;
     mg_drop_exchange(mg);
     for (ThreadCtx *c : mg->ctx) delete c;   // ~ThreadCtx gives back the scanner, streams, events and buffers
-    cudaSetDevice(keep);
     delete mg;
 }
 
@@ -137,10 +127,9 @@ int bmx_mg_search(bmx_mg *mg, const char *text, int64_t n, const char *pat, int3
                   uint64_t *count_out, uint64_t *shard_counts)
 {
     if (!mg || !count_out || !pat) return fail(BMX_E_BADARG, "bmx_mg_search: NULL argument");
-    if (n < 0 || (!text && n > 0)) return fail(BMX_E_BADARG, "bmx_mg_search: bad text (n=%lld)", (long long)n);
+    if (int rc = check_text(text, n, "bmx_mg_search")) return rc;
     if (pos_cap < 0) return fail(BMX_E_BADARG, "pos_cap < 0");
-    if (m <= 0 || m > BMX_MAX_PATTERN)
-        return fail(BMX_E_BADARG, "pattern length %d outside 1..%d (an empty pattern is rejected)", m, BMX_MAX_PATTERN);
+    if (int rc = check_pattern(m)) return rc;
     const int R = (int)mg->devices.size();
     *count_out = 0;
     for (int r = 0; r < R && shard_counts; ++r) shard_counts[r] = 0;
@@ -187,8 +176,7 @@ int bmx_mg_search(bmx_mg *mg, const char *text, int64_t n, const char *pat, int3
         if (shard_counts) shard_counts[r] = sh[(size_t)r].count;
     }
     // gather: shard lists are ascending and shards are ordered, so concatenation is the sorted result
-    int keep = 0;
-    cudaGetDevice(&keep);
+    ScopedDevice keep;
     int64_t off = 0;
     for (int r = 0; r < R; ++r) {
         Shard &s = sh[(size_t)r];
@@ -211,7 +199,6 @@ int bmx_mg_search(bmx_mg *mg, const char *text, int64_t n, const char *pat, int3
             err = "stream synchronisation failed";
         }
     }
-    cudaSetDevice(keep);
     if (rc != BMX_OK) return fail(rc, "bmx_mg_search: %s", err.c_str());
     *count_out = total;
     return BMX_OK;
@@ -223,15 +210,13 @@ int bmx_mg_search_device(bmx_mg *mg, const void *const *d_text, const int64_t *n
 {
     if (!mg || !d_text || !n || !pos_base || !pat || !count_out) return fail(BMX_E_BADARG, "bmx_mg_search_device: NULL argument");
     if (pos_cap < 0) return fail(BMX_E_BADARG, "pos_cap < 0");
-    if (m <= 0 || m > BMX_MAX_PATTERN)
-        return fail(BMX_E_BADARG, "pattern length %d outside 1..%d (an empty pattern is rejected)", m, BMX_MAX_PATTERN);
+    if (int rc = check_pattern(m)) return rc;
     const int R = (int)mg->devices.size();
     for (int r = 0; r < R; ++r)
         if (n[r] < 0 || (!d_text[r] && n[r] > 0)) return fail(BMX_E_BADARG, "bmx_mg_search_device: bad shard %d (n=%lld)", r, (long long)n[r]);
     *count_out = 0;
     const bool want_pos = d_pos_out != nullptr && pos_cap > 0;
-    int keep = 0;
-    cudaGetDevice(&keep);
+    ScopedDevice keep;
     int rc = BMX_OK;
     std::vector<uint64_t> counts((size_t)R, 0);
     uint64_t total = 0;
@@ -243,7 +228,7 @@ int bmx_mg_search_device(bmx_mg *mg, const void *const *d_text, const int64_t *n
         for (int r = 0; r < R && rc == BMX_OK; ++r) {   // every launch is asynchronous: one host thread feeds all GPUs
             ThreadCtx *c = mg->ctx[(size_t)r];
             cudaSetDevice(mg->devices[(size_t)r]);
-            if ((rc = ensure_streams(*c, mg->devices[(size_t)r], 1)) != BMX_OK) break;
+            if ((rc = ensure_streams(*c, 1)) != BMX_OK) break;
             if ((rc = bmx_scanner_set_pattern(c->scanner, pat, m, BMX_VARIANT_AUTO, c->scan_stream)) != BMX_OK) break;
             if ((rc = bmx_scanner_begin(c->scanner, want_pos ? mg->d_local_pos[(size_t)r] : nullptr, local_cap, c->scan_stream)) != BMX_OK) break;
             if ((rc = bmx_scanner_scan(c->scanner, d_text[r], n[r], pos_base[r], c->scan_stream)) != BMX_OK) break;
@@ -272,7 +257,6 @@ int bmx_mg_search_device(bmx_mg *mg, const void *const *d_text, const int64_t *n
         if (need <= kMgHeadCap + mg->xchg_tail_cap) break;
         tail_cap = ((need - kMgHeadCap) + 4095) & ~int64_t(4095);
     }
-    cudaSetDevice(keep);
     if (rc != BMX_OK) return rc;
     *count_out = total;
     for (int r = 0; r < R && shard_counts; ++r) shard_counts[r] = counts[(size_t)r];

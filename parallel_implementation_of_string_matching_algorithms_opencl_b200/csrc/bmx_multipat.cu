@@ -40,21 +40,6 @@ struct MultiImage {
     uint32_t hmul = 0, hmul2 = 0;
 };
 
-uint32_t le_word(const unsigned char *p, int nbytes)
-{
-    uint32_t w = 0;
-    for (int i = 0; i < nbytes && i < 4; ++i) w |= (uint32_t)p[i] << (8 * i);
-    return w;
-}
-
-bool multi_eligible(int32_t npat, const int32_t *ms)
-{
-    if (npat < 1 || npat > kMultiMaxPatterns) return false;
-    for (int32_t k = 0; k < npat; ++k)
-        if (ms[k] < 7 || ms[k] > kHaloSmemMax) return false;
-    return true;
-}
-
 void build_multi_image(int32_t npat, const char *const *pats, const int32_t *ms, MultiImage *im)
 {
     im->m_min = *std::min_element(ms, ms + npat);
@@ -62,8 +47,8 @@ void build_multi_image(int32_t npat, const char *const *pats, const int32_t *ms,
     // one gram length for all patterns and residues: q = min(12, m_min - 3) bytes = 4 + q2 (second word) + q3 (third word)
     const int q = std::min(12, im->m_min - 3);
     const int q2 = std::min(4, q - 4), q3 = std::max(0, q - 8);
-    im->hmul = q2 >= 4 ? kHashMul : (q2 == 0 ? 0u : (kHashMul << (32 - 8 * q2)));   // the shift drops the bytes beyond the gram
-    im->hmul2 = q3 >= 4 ? kHashMul2 : (q3 == 0 ? 0u : (kHashMul2 << (32 - 8 * q3)));
+    im->hmul = gram_multiplier(kHashMul, q2);
+    im->hmul2 = gram_multiplier(kHashMul2, q3);
     auto align16 = [](size_t v) { return (v + 15) & ~size_t(15); };
     im->off_table = (size_t)kMultiBitmapWords * 4;
     im->off_dir = im->off_table + (size_t)kMultiSlots * 8;
@@ -138,11 +123,6 @@ __global__ void __launch_bounds__(kSplitThreads) multi_split_kernel(const int64_
     if (tid == 0) split_counts[k] = running;
 }
 
-int64_t first_union_cap(int64_t n, int32_t m_min, int64_t want)
-{
-    return std::max<int64_t>(0, std::min<int64_t>({want, n - m_min + 1, std::max<int64_t>(int64_t(1) << 20, n / 64)}));
-}
-
 }  // namespace
 
 namespace bmx {
@@ -187,16 +167,18 @@ int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, in
     s->proto.multi_blob_smem = blob_bytes <= (size_t)kPatSmemMax * 4 ? (uint32_t)blob_bytes : 0u;   // SmemCtl::good holds kPatSmemMax ints
     s->m = im.m_min;
     s->m_halo = im.m_max;
-    const int keep_timing = s->timing_level;
-    s->timing_level = 0;
+    ScopedTiming timing(s, 0);
 
-    int64_t cap_u = any_out ? first_union_cap(n, im.m_min, want) : 0;
-    if (any_out && (int64_t)(c.pos.cap / 8) > cap_u) cap_u = std::min<int64_t>(want, (int64_t)(c.pos.cap / 8));
+    // from here on every failure breaks out of the loop, so that the scanner leaves multi-pattern mode below
+    int64_t cap_u = any_out ? first_pos_room(c, n, im.m_min, want) : 0;
     std::vector<unsigned long long> h_counts((size_t)2 * kMultiMaxPatterns, 0);
     int rc = BMX_OK;
     for (int pass = 0; pass < 2 && rc == BMX_OK; ++pass) {
         if (cap_u > 0 && (rc = ensure_buf(c, c.pos, (size_t)cap_u * 8)) != BMX_OK) break;
-        if (pass > 0) BMX_CUDA(cudaMemsetAsync(d_im + im.off_counts, 0, (size_t)kMultiMaxPatterns * 8, st));
+        if (pass > 0 && cudaMemsetAsync(d_im + im.off_counts, 0, (size_t)kMultiMaxPatterns * 8, st) != cudaSuccess) {
+            rc = fail(BMX_E_CUDA, "bmx_search_multi: %s", cudaGetErrorString(cudaGetLastError()));
+            break;
+        }
         int64_t *U = cap_u > 0 ? static_cast<int64_t *>(c.pos.p) : nullptr;
         if ((rc = bmx_scanner_begin(s, U, cap_u, st)) != BMX_OK) break;
         if ((rc = bmx_scanner_scan(s, d_text, n, 0, st)) != BMX_OK) break;
@@ -224,7 +206,6 @@ int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, in
         if (!short_list || (int64_t)ucount <= cap_u) break;
         cap_u = (int64_t)ucount;   // the union list was cut short before some pattern had its share: room for all of it
     }
-    s->timing_level = keep_timing;
     s->m_halo = 0;
     s->m = 0;   // the scanner has no single pattern until the next set_pattern
     if (rc != BMX_OK) return rc;
@@ -232,7 +213,13 @@ int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, in
     return BMX_OK;
 }
 
-bool multi_set_eligible(int32_t npat, const int32_t *ms) { return multi_eligible(npat, ms); }
+bool multi_eligible(int32_t npat, const int32_t *ms)
+{
+    if (npat < 1 || npat > kMultiMaxPatterns) return false;
+    for (int32_t k = 0; k < npat; ++k)
+        if (ms[k] < 7 || ms[k] > kHaloSmemMax) return false;
+    return true;
+}
 
 }  // namespace bmx
 
@@ -241,20 +228,11 @@ extern "C" {
 int bmx_search_multi_device(const void *d_text, int64_t n, int32_t npat, const char *const *pats, const int32_t *ms,
                             int64_t *const *d_pos_out, const int64_t *pos_cap, uint64_t *counts, void *stream)
 {
-    if (npat < 0 || (npat > 0 && (!pats || !ms || !counts))) return fail(BMX_E_BADARG, "bmx_search_multi_device: NULL argument or npat < 0");
-    if (n < 0 || (!d_text && n > 0)) return fail(BMX_E_BADARG, "bmx_search_multi_device: bad text (n=%lld)", (long long)n);
-    for (int32_t k = 0; k < npat; ++k) {
-        if (!pats[k] || ms[k] <= 0 || ms[k] > BMX_MAX_PATTERN)
-            return fail(BMX_E_BADARG, "pattern %d: length %d outside 1..%d or NULL (an empty pattern is rejected)", k, ms[k], BMX_MAX_PATTERN);
-        if (d_pos_out && d_pos_out[k] && (!pos_cap || pos_cap[k] < 0)) return fail(BMX_E_BADARG, "pattern %d: pos_cap < 0 or missing", k);
-        counts[k] = 0;
-    }
+    if (int rc = check_text(d_text, n, "bmx_search_multi_device")) return rc;
+    if (int rc = check_pattern_set(npat, pats, ms, d_pos_out, pos_cap, counts, "bmx_search_multi_device")) return rc;
     if (npat == 0 || n == 0) return BMX_OK;
-    int device = 0;
-    if (int rc = check_device(0)) return rc;
-    BMX_CUDA(cudaGetDevice(&device));
     ThreadCtx *c = nullptr;
-    if (int rc = get_ctx(device, &c)) return rc;
+    if (int rc = current_ctx(&c)) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (multi_eligible(npat, ms))
         return multi_scan_resident(*c, static_cast<const unsigned char *>(d_text), n, npat, pats, ms, d_pos_out, pos_cap, counts, st);
@@ -263,11 +241,8 @@ int bmx_search_multi_device(const void *d_text, int64_t n, int32_t npat, const c
     for (int32_t k = 0; k < npat; ++k) {
         if (n < ms[k]) continue;
         int64_t *out = d_pos_out ? d_pos_out[k] : nullptr;
-        int rc = bmx_scanner_set_pattern(c->scanner, pats[k], ms[k], BMX_VARIANT_AUTO, st);
-        if (rc == BMX_OK) rc = bmx_scanner_begin(c->scanner, out, out ? pos_cap[k] : 0, st);
-        if (rc == BMX_OK) rc = bmx_scanner_scan(c->scanner, d_text, n, 0, st);
-        if (rc == BMX_OK) rc = bmx_scanner_finish(c->scanner, &counts[k], nullptr, st);
-        if (rc != BMX_OK) return rc;
+        if (int rc = search_once(c->scanner, pats[k], ms[k], BMX_VARIANT_AUTO, d_text, n, 0, out, out ? pos_cap[k] : 0, &counts[k], nullptr, st))
+            return rc;
     }
     return BMX_OK;
 }

@@ -44,7 +44,7 @@
 #include <mutex>
 #include <utility>
 
-#include "bmx_internal.h"
+#include "bmx_ctx.h"
 
 namespace bmx {
 
@@ -1384,19 +1384,6 @@ __global__ void export_result_kernel(const unsigned long long *count, const int6
 // ---------------------------------------------------------------------------------------------
 // Host: filter choice, planning, launch
 // ---------------------------------------------------------------------------------------------
-static int env_int(const char *name, int fallback)
-{
-    const char *v = getenv(name);
-    return (v && *v) ? atoi(v) : fallback;
-}
-
-static uint32_t le_word(const unsigned char *p, int nbytes)
-{
-    uint32_t w = 0;
-    for (int i = 0; i < nbytes && i < 4; ++i) w |= (uint32_t)p[i] << (8 * i);
-    return w;
-}
-
 Filter choose_filter(int requested_variant, const unsigned char *pat, int32_t m)
 {
     // AUTO, and QGRAM for m < 7: thresholds from the measured table in DESIGN.md (profiles/variants_r01.json)
@@ -1434,7 +1421,7 @@ void fill_filter_constants(Filter filter, const unsigned char *pat, int32_t m, S
         // residue r (pattern byte r on a word boundary) can use min(8, m - r) pattern bytes
         for (int r = 0; r < 4; ++r) {
             const int q2 = std::min(m - r, 8) - 4;   // bytes taken from the second word
-            a->hmulr[r] = q2 >= 4 ? kHashMul : (q2 == 0 ? 0u : (kHashMul << (32 - 8 * q2)));
+            a->hmulr[r] = gram_multiplier(kHashMul, q2);
             a->f[r] = le_word(pat + r, 4) + a->hmulr[r] * le_word(pat + r + 4, q2);
         }
         a->hmul = a->hmulr[3];
@@ -1488,14 +1475,12 @@ static int device_info(int device, int *sm_count, int *smem_optin, int *smem_sm,
             cudaDeviceGetAttribute(&q.smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) != cudaSuccess ||
             cudaDeviceGetAttribute(&q.smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, device) != cudaSuccess)
             return fail(BMX_E_CUDA, "cudaDeviceGetAttribute: %s", cudaGetErrorString(cudaGetLastError()));
-        int cur = 0;
-        cudaGetDevice(&cur);
-        if (cur != device) cudaSetDevice(device);
+        ScopedDevice keep;   // the occupancy query reads the current device
+        cudaSetDevice(device);
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&q.expand_per_sm, expand_kernel, kExpandThreads, 0) != cudaSuccess || q.expand_per_sm < 1) {
             (void)cudaGetLastError();
             q.expand_per_sm = 2;
         }
-        if (cur != device) cudaSetDevice(cur);
         di = q;
     }
     if (sm_count) *sm_count = di.sm_count;

@@ -109,6 +109,61 @@ def test_bad_arguments_are_rejected_without_touching_a_gpu(bmx):
     assert lib.bmx_search_partitions(b"abcab", b"ab", se, ans, wrong_gs, None, 2, 1) == E.BMX_E_TABLES
     assert lib.bmx_partition_words(b"a b", 3, 0, se) == E.BMX_E_BADARG
 
+    # The other entry points, one bad argument each.  BADARG alone where the check comes before the device lookup;
+    # BADARG or NODEVICE where it comes after (a machine without a GPU stops at the lookup).
+    either = (E.BMX_E_BADARG, E.BMX_E_NODEVICE)
+    first = ctypes.c_int64()
+    assert lib.bmx_search_device_ex(None, -1, b"a", 1, 0, None, 0, ctypes.byref(cnt), 0, None, None) == E.BMX_E_BADARG
+    assert lib.bmx_search_device_ex(None, 0, b"a", 1, 0, None, 0, None, 0, None, None) == E.BMX_E_BADARG
+    assert lib.bmx_search_device_ex(None, 0, b"a", 1, 0, None, -1, ctypes.byref(cnt), 0, None, None) == E.BMX_E_BADARG
+    assert lib.bmx_search_device_ex(None, 0, b"", 0, 0, None, 0, ctypes.byref(cnt), 0, None, None) in either
+    assert lib.bmx_find_first_device(None, -1, b"a", 1, ctypes.byref(first), None) == E.BMX_E_BADARG
+    assert lib.bmx_find_first_device(None, 0, b"a", 1, None, None) == E.BMX_E_BADARG
+    assert lib.bmx_find_first_device(None, 0, b"", 0, ctypes.byref(first), None) in either
+    assert lib.bmx_find_first(b"abc", -1, b"a", 1, ctypes.byref(first)) == E.BMX_E_BADARG
+    assert lib.bmx_find_first(b"abc", 3, b"a", 1, None) == E.BMX_E_BADARG
+    assert lib.bmx_find_first(b"abc", 3, b"", 0, ctypes.byref(first)) == E.BMX_E_BADARG
+
+    pats = (ctypes.c_char_p * 2)(b"ab", None)   # a NULL pattern in the set
+    ms = (ctypes.c_int32 * 2)(2, 2)
+    ms0 = (ctypes.c_int32 * 2)(2, 0)
+    good_pats = (ctypes.c_char_p * 2)(b"ab", b"cd")
+    counts = (ctypes.c_uint64 * 2)()
+    multi_host = lambda *a: lib.bmx_search_multi(0, *a)              # noqa: E731
+    multi_device = lambda *a: lib.bmx_search_multi_device(*a, None)  # noqa: E731
+    for fn in (multi_host, multi_device):
+        assert fn(b"abcd", 4, 2, pats, ms, None, None, counts) == E.BMX_E_BADARG
+        assert fn(b"abcd", 4, 2, good_pats, ms0, None, None, counts) == E.BMX_E_BADARG
+        assert fn(b"abcd", -1, 2, good_pats, ms, None, None, counts) == E.BMX_E_BADARG
+        assert fn(b"abcd", 4, -1, good_pats, ms, None, None, counts) == E.BMX_E_BADARG
+        assert fn(b"abcd", 4, 2, good_pats, ms, None, None, None) == E.BMX_E_BADARG
+
+    # a zeroed block stands in for a bmx_mg handle: these calls reject their arguments before they read it
+    mg = ctypes.create_string_buffer(256)
+    shard_counts = (ctypes.c_uint64 * 1)()
+    assert lib.bmx_mg_search(None, b"abc", 3, b"a", 1, None, 0, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+    assert lib.bmx_mg_search(mg, b"abc", -1, b"a", 1, None, 0, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+    assert lib.bmx_mg_search(mg, b"abc", 3, b"", 0, None, 0, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+    assert lib.bmx_mg_search(mg, b"abc", 3, b"a", 1, None, -1, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+    texts = (ctypes.c_void_p * 1)()
+    lens = (ctypes.c_int64 * 1)(3)
+    bases = (ctypes.c_int64 * 1)(0)
+    assert lib.bmx_mg_search_device(None, texts, lens, bases, b"a", 1, None, 0, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+    assert lib.bmx_mg_search_device(mg, None, lens, bases, b"a", 1, None, 0, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+    assert lib.bmx_mg_search_device(mg, texts, lens, bases, b"", 0, None, 0, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+    assert lib.bmx_mg_search_device(mg, texts, lens, bases, b"a", 1, None, -1, ctypes.byref(cnt), shard_counts) == E.BMX_E_BADARG
+
+    handle = ctypes.c_void_p()
+    assert lib.bmx_exchange_create(0, 0, 1, 0, 0, 0, 2, None) == E.BMX_E_BADARG
+    assert lib.bmx_exchange_create(0, 0, 0, 0, 0, 0, 2, ctypes.byref(handle)) == E.BMX_E_BADARG   # world 0
+    assert lib.bmx_exchange_create(0, 1, 1, 0, 0, 0, 2, ctypes.byref(handle)) == E.BMX_E_BADARG   # rank >= world
+    assert lib.bmx_exchange_create(0, 0, 1, 0, -1, 0, 2, ctypes.byref(handle)) == E.BMX_E_BADARG  # head_cap < 0
+    assert lib.bmx_exchange_create(0, 0, 1, 0, 0, 0, 1, ctypes.byref(handle)) == E.BMX_E_BADARG   # depth < 2
+    assert lib.bmx_exchange_create(-1, 0, 1, 0, 0, 0, 2, ctypes.byref(handle)) in either
+    assert lib.bmx_scanner_create(0, None) == E.BMX_E_BADARG
+    assert lib.bmx_scanner_create(-1, ctypes.byref(handle)) in either
+    assert not handle.value
+
 
 def test_no_cpu_fallback(bmx):
     """Without a CUDA device a scan must fail loudly, never quietly compute on the host."""

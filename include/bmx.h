@@ -182,6 +182,35 @@ int bmx_search_partitions(const char *text, const char *pat, const int32_t *se, 
                           const int32_t *gs, const int32_t *bs, int32_t m, int32_t nparts);
 
 /*
+ * Many ranges of one text in one call -- generalises the kernel entry search(text, pattern, se, ans, ...)
+ * (kernel1.cl:1, occurrences lying fully inside each range, no halo) with the ranges the reference builds at
+ * BoyreMoore.cpp:119-141, to any number of half-open ranges, with positions.  Range d = [begin[d], end[d]),
+ * 0 <= begin[d] <= end[d] <= n; ranges may come in any order, overlap or be empty.
+ *   counts[d]  = number of p with begin[d] <= p, p + m <= end[d], text[p..p+m) == pat: exactly what bmx_search
+ *                returns for the text + begin[d] of length end[d] - begin[d] (a match across a range edge counts
+ *                in no range);
+ *   offsets[d] = counts[0] + ... + counts[d-1], offsets[nranges] = the total (nranges + 1 entries, always exact);
+ *   pos_out    = the ranges' position lists one after the other (CSR): pos_out[offsets[d] .. offsets[d+1]) holds
+ *                range d's match starts RELATIVE TO begin[d], ascending.  Only the first min(total, pos_cap)
+ *                entries are written; pos_out == NULL is counts only.
+ * A ragged batch held as values + offsets o[0..D] is passed as begin = o, end = o + 1, without a copy.
+ * The covered bytes are scanned once with positions and every range is answered from that one ascending list
+ * (binary searches + a gather), so the per-call cost is paid once per batch, not once per range.
+ * bmx_search_ranges: host text, ranges and outputs; ranges are checked on the host (BMX_E_BADARG names the first
+ * bad one); only [min begin, max end) crosses PCIe.  Synchronous.
+ * bmx_search_ranges_device: d_text, d_begin, d_end, d_pos_out, d_counts, d_offsets are DEVICE memory on the current
+ * device; the total goes to the host (*total_out).  A range outside [0, n] is found on the device and reported as
+ * BMX_E_BADARG (never a fault).  Synchronous on `stream`.
+ */
+int bmx_search_ranges(int device, const char *text, int64_t n, int64_t nranges,
+                      const int64_t *begin, const int64_t *end, const char *pat, int32_t m,
+                      int64_t *pos_out, int64_t pos_cap, uint64_t *counts, int64_t *offsets /* nranges+1 */);
+int bmx_search_ranges_device(const void *d_text, int64_t n, int64_t nranges,
+                             const int64_t *d_begin, const int64_t *d_end, const char *pat, int32_t m,
+                             int64_t *d_pos_out, int64_t pos_cap, uint64_t *d_counts, int64_t *d_offsets,
+                             uint64_t *total_out, void *stream);
+
+/*
  * The reference's host-side word partitioner -- replaces BoyreMoore.cpp:94-141.  Splits
  * text[0..n) (up to the first NUL, like the reference's strcpy'd copy, :89-90) on single spaces
  * into nparts inclusive byte ranges of equal word count: se[2*p], se[2*p+1].  The space between

@@ -33,6 +33,7 @@ EXPORTS = [
     "bmx_scanner_scan", "bmx_scanner_finish", "bmx_scanner_export_result", "bmx_scanner_set_timing", "bmx_mg_create", "bmx_mg_destroy", "bmx_mg_device_count", "bmx_mg_search", "bmx_synth_fill_device", "bmx_partition_words",
     "bmx_mg_search_device", "bmx_exchange_create", "bmx_exchange_destroy", "bmx_exchange_handle", "bmx_exchange_connect",
     "bmx_exchange_connect_local", "bmx_exchange_post", "bmx_exchange_collect", "bmx_exchange_wait", "bmx_release_memory", "bmx_search_multi_device",
+    "bmx_search_ranges", "bmx_search_ranges_device",
 ]
 
 
@@ -95,6 +96,10 @@ def load() -> ctypes.CDLL:
     lib.bmx_find_first_device.argtypes = [c_void_p, c_int64, c_char_p, c_int32, POINTER(c_int64), c_void_p]
     lib.bmx_search_partitions.argtypes = [c_void_p, c_char_p, POINTER(c_int32), POINTER(c_int32),
                                           POINTER(c_int32), POINTER(c_int32), c_int32, c_int32]
+    lib.bmx_search_ranges.argtypes = [c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_char_p, c_int32,
+                                      c_void_p, c_int64, c_void_p, c_void_p]
+    lib.bmx_search_ranges_device.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_char_p, c_int32,
+                                             c_void_p, c_int64, c_void_p, c_void_p, POINTER(c_uint64), c_void_p]
     lib.bmx_scanner_create.argtypes = [c_int, POINTER(c_void_p)]
     lib.bmx_scanner_destroy.argtypes = [c_void_p]
     lib.bmx_scanner_destroy.restype = None

@@ -89,6 +89,12 @@ inline int64_t first_pos_room(const ThreadCtx &c, int64_t n, int32_t m, int64_t 
 int ingest_shard(ThreadCtx &ctx, int device, const char *text, int64_t n, const char *pat, int32_t m, int64_t pos_base,
                  int64_t want_cap, uint64_t *count, int64_t *dev_cap);
 
+// Per-range counts, offsets and positions of host ranges over a host text (bmx_ranges.cu).  The ranges are checked
+// (inside [0, n], begin <= end) and cover [lo, hi); counts / offsets / pos_out are host memory.
+int search_ranges_host(ThreadCtx &c, const char *text, int64_t n, int64_t nranges, const int64_t *begin, const int64_t *end,
+                       int64_t lo, int64_t hi, const char *pat, int32_t m, int64_t *pos_out, int64_t pos_cap, uint64_t *counts,
+                       int64_t *offsets);
+
 // K patterns in one pass over device-resident text (bmx_multipat.cu)
 bool multi_eligible(int32_t npat, const int32_t *ms);
 int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, int32_t npat, const char *const *pats,

@@ -502,34 +502,20 @@ int bmx_search_partitions(const char *text, const char *pat, const int32_t *se, 
 
     ThreadCtx *c = nullptr;
     if (int rc = current_ctx(&c)) return rc;
-    if (int rc = ensure_streams(*c, 1)) return rc;
-    cudaStream_t st = c->scan_stream;
-    // One work-item of the reference = one count-only scan of its inclusive range (occurrences lying fully
-    // inside it, kernel1.cl:15,19): no position list, so no memory proportional to the text beyond the text.
-    if (int rc = ensure_buf(*c, c->text, (size_t)span + 16)) return rc;
-    if (int rc = ensure_buf(*c, c->misc, (size_t)nparts * 8)) return rc;
-    unsigned char *d_text = static_cast<unsigned char *>(c->text.p);
-    unsigned long long *d_counts = static_cast<unsigned long long *>(c->misc.p);
-    BMX_CUDA(cudaMemsetAsync(d_counts, 0, (size_t)nparts * 8, st));
-    BMX_CUDA(cudaMemcpyAsync(d_text, text + lo, (size_t)span, cudaMemcpyHostToDevice, st));
-    if (int rc = bmx_scanner_set_pattern(c->scanner, pat, m, BMX_VARIANT_AUTO, st)) return rc;
-    ScopedTiming timing(c->scanner, 0);
-    int rc = BMX_OK;
-    for (int32_t id = 0; id < nparts && rc == BMX_OK; ++id) {
-        const int64_t a = se[2 * id], len = (int64_t)se[2 * id + 1] - a + 1;
-        if (len < m) continue;
-        rc = bmx_scanner_begin(c->scanner, nullptr, 0, st);
-        if (rc == BMX_OK) rc = bmx_scanner_scan(c->scanner, d_text + (a - lo), len, a, st);
-        if (rc == BMX_OK && cudaMemcpyAsync(d_counts + id, result_slot(c->scanner), 8, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
-            rc = fail(BMX_E_CUDA, "bmx_search_partitions: %s", cudaGetErrorString(cudaGetLastError()));
+    // One work-item of the reference = the occurrences lying fully inside its inclusive range (kernel1.cl:15,19):
+    // range [s, e + 1) of the ranges search, which scans the covered bytes [lo, hi] once with positions and
+    // answers every range from that one list (bmx_ranges.cu).  A range with e < s counts 0: it becomes empty.
+    std::vector<int64_t> begin((size_t)nparts), end((size_t)nparts), offsets((size_t)nparts + 1);
+    std::vector<uint64_t> counts((size_t)nparts, 0);
+    for (int32_t id = 0; id < nparts; ++id) {
+        const int64_t s = se[2 * id], e = (int64_t)se[2 * id + 1] + 1;
+        begin[(size_t)id] = e < s ? lo : s;
+        end[(size_t)id] = e < s ? lo : e;
     }
-    std::vector<unsigned long long> h_counts((size_t)nparts, 0);
-    if (rc == BMX_OK && cudaMemcpyAsync(h_counts.data(), d_counts, (size_t)nparts * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess)
-        rc = fail(BMX_E_CUDA, "bmx_search_partitions: %s", cudaGetErrorString(cudaGetLastError()));
-    const cudaError_t e = cudaStreamSynchronize(st);
-    if (rc == BMX_OK && e != cudaSuccess) rc = fail(BMX_E_CUDA, "bmx_search_partitions: %s", cudaGetErrorString(e));
-    if (rc != BMX_OK) return rc;
-    for (int32_t id = 0; id < nparts; ++id) ans[id] = (int32_t)h_counts[(size_t)id];
+    if (int rc = search_ranges_host(*c, text, hi + 1, nparts, begin.data(), end.data(), lo, hi + 1, pat, m, nullptr, 0,
+                                    counts.data(), offsets.data()))
+        return rc;
+    for (int32_t id = 0; id < nparts; ++id) ans[id] = (int32_t)counts[(size_t)id];
     return BMX_OK;
 }
 

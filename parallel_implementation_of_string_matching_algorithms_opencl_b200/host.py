@@ -251,6 +251,83 @@ def search_partitions(text, pattern, se, gs=None, bs=None) -> np.ndarray:
     return ans
 
 
+def search_ranges(text, pattern, begin, end, max_positions: int | None = None, device: int | None = None):
+    """Many ranges of one HOST text in one pass (bmx_search_ranges) -- the kernel entry `search` (kernel1.cl:1)
+    for any number of half-open ranges [begin[d], end[d]), with positions.  Returns (counts, offsets, positions):
+
+        counts[d]     matches lying fully inside range d (= search(text[begin[d]:end[d]], pattern)[0])
+        offsets       nranges + 1 entries, offsets[d] = counts[:d].sum(), offsets[-1] = total
+        positions     range d's starts, RELATIVE TO begin[d], at positions[offsets[d]:offsets[d+1]] (the first
+                      min(total, max_positions) entries of that concatenation)
+
+    max_positions=None: room for all (grown like search()); 0: counts only (positions is empty).
+    A ragged batch held as values + offsets o is one call:
+
+        counts, offs, pos = search_ranges(values, pattern, begin=o[:-1], end=o[1:])
+    """
+    lib = _lib.load()
+    pat = _as_bytes(pattern)
+    ptr, n, keep = _host_text(text)
+    b = np.ascontiguousarray(begin, dtype=np.int64).reshape(-1)
+    e = np.ascontiguousarray(end, dtype=np.int64).reshape(-1)
+    if b.size != e.size:
+        raise ValueError("begin and end must have the same length")
+    if device is None:
+        import torch
+        device = torch.cuda.current_device() if torch.cuda.is_available() else 0
+    d = b.size
+    counts = np.zeros(d, dtype=np.uint64)
+    offsets = np.zeros(d + 1, dtype=np.int64)
+    open_ended = max_positions is None
+    cap = _first_cap(n, len(pat)) if open_ended else int(max_positions)
+    while True:
+        pos = np.empty(cap, dtype=np.int64)
+        check(lib.bmx_search_ranges(device, ptr, n, d, b.ctypes.data if d else None, e.ctypes.data if d else None, pat, len(pat),
+                                    pos.ctypes.data if cap else None, cap, counts.ctypes.data if d else None, offsets.ctypes.data))
+        total = int(offsets[-1])
+        if not open_ended or total <= cap:
+            break
+        cap = total
+    del keep
+    return counts, offsets, pos[: min(total, cap)]
+
+
+def search_ranges_device(text, pattern, begin, end, max_positions: int = 0, stream=None):
+    """search_ranges() for CUDA tensors (bmx_search_ranges_device): a contiguous uint8 text and int64 begin / end on
+    the same device.  Returns (counts int64, offsets int64 [nranges + 1], positions or None) as CUDA tensors;
+    positions is the filled prefix of a tensor of max_positions entries (0 = counts only).  Ragged batch:
+
+        counts, offs, pos = search_ranges_device(values, pattern, offs_in[:-1], offs_in[1:], max_positions=k)
+
+    A range outside [0, len(text)] raises BmxError (BMX_E_BADARG); the library stays usable.
+    """
+    import torch
+
+    lib = _lib.load()
+    pat = _as_bytes(pattern)
+    if not text.is_cuda or text.dtype != torch.uint8 or not text.is_contiguous():
+        raise TypeError("search_ranges_device() needs a contiguous CUDA uint8 tensor")
+    for t in (begin, end):
+        if not t.is_cuda or t.dtype != torch.int64 or t.dim() != 1 or t.device != text.device:
+            raise TypeError("begin / end must be 1-D CUDA int64 tensors on the text's device")
+    if begin.numel() != end.numel():
+        raise ValueError("begin and end must have the same length")
+    begin, end = begin.contiguous(), end.contiguous()
+    n, d, cap = text.numel(), begin.numel(), int(max_positions)
+    with torch.cuda.device(text.device):
+        counts = torch.empty(d, dtype=torch.int64, device=text.device)
+        offsets = torch.empty(d + 1, dtype=torch.int64, device=text.device)
+        pos = torch.empty(cap, dtype=torch.int64, device=text.device) if cap else None
+        s = stream if stream is not None else torch.cuda.current_stream(text.device)
+        total = c_uint64(0)
+        check(lib.bmx_search_ranges_device(c_void_p(text.data_ptr() if n else 0), n, d, c_void_p(begin.data_ptr() if d else 0),
+                                           c_void_p(end.data_ptr() if d else 0), pat, len(pat),
+                                           c_void_p(pos.data_ptr()) if cap else None, cap,
+                                           c_void_p(counts.data_ptr() if d else 0), c_void_p(offsets.data_ptr()),
+                                           ctypes.byref(total), c_void_p(s.cuda_stream)))
+    return counts, offsets, None if pos is None else pos[: min(total.value, cap)]
+
+
 class Scanner:
     """Reusable scanner (bmx_scanner_*): pattern block + look-back scratch kept across scans."""
 

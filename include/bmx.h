@@ -52,6 +52,19 @@ typedef enum bmx_variant {
     BMX_VARIANT_SHIFTAND = 3  /* m <= 32: bit-parallel Shift-And (the Shift-Or family) */
 } bmx_variant;
 
+/*
+ * Case-insensitive search (grep -i over ASCII): OR'ed into the `variant` argument of bmx_search_ex,
+ * bmx_search_device_ex and bmx_scanner_set_pattern.  Position p then matches when fold(text[p+i]) == fold(pat[i])
+ * for every i < m, where fold maps 'A'..'Z' (0x41-0x5A) to 'a'..'z' and leaves every other byte value alone,
+ * 0x80-0xFF included (Python's bytes.lower(); no Unicode or locale folding).  The result -- count, positions,
+ * ordering, pos_cap truncation, pos_base -- is exactly the exact search's result for lower(text) and lower(pat).
+ * The caller's text is never written: the scan kernel folds its own shared-memory copy of each tile.
+ * An unknown bit in `variant`, or an unknown base variant with the flag, is BMX_E_BADARG.  A pattern without an
+ * ASCII letter matches the same set either way: the flag is then dropped and the exact kernels run.
+ * bmx_stats.variant reports `variant | BMX_IGNORE_CASE` exactly when the case-folding kernels ran.
+ */
+#define BMX_IGNORE_CASE 0x100
+
 /* Per-call measurements filled by the *_ex / scanner calls (all optional). */
 typedef struct bmx_stats {
     float device_ms;       /* CUDA-event time of the scan + expand kernel(s) on the launching stream */
@@ -109,7 +122,7 @@ int bmx_search(const char *text, int64_t n, const char *pat, int32_t m,
                int64_t *pos_out, int64_t pos_cap, uint64_t *count_out);
 
 /* As bmx_search, on an explicit device, with variant choice and measurements.  CUDA events are recorded only
- * when stats is non-NULL (they cost ~15 us per call). */
+ * when stats is non-NULL (they cost ~15 us per call).  variant may carry BMX_IGNORE_CASE. */
 int bmx_search_ex(int device, const char *text, int64_t n, const char *pat, int32_t m,
                   int64_t *pos_out, int64_t pos_cap, uint64_t *count_out,
                   int32_t variant, bmx_stats *stats);
@@ -161,7 +174,7 @@ int bmx_find_first_device(const void *d_text, int64_t n, const char *pat, int32_
                           void *stream);
 
 /* As bmx_search_device with: pos_base added to every reported position (multi-GPU shards report
- * global offsets), explicit variant, full measurements. */
+ * global offsets), explicit variant (may carry BMX_IGNORE_CASE), full measurements. */
 int bmx_search_device_ex(const void *d_text, int64_t n, const char *pat, int32_t m,
                          int64_t pos_base, int64_t *d_pos_out, int64_t pos_cap,
                          uint64_t *count_out, int32_t variant, bmx_stats *stats, void *stream);
@@ -231,7 +244,8 @@ typedef struct bmx_scanner bmx_scanner;
 int bmx_scanner_create(int device, bmx_scanner **out);
 void bmx_scanner_destroy(bmx_scanner *s);
 
-/* Builds the tables (bmx_build_tables) and uploads the pattern block on `stream`. */
+/* Builds the tables (bmx_build_tables) and uploads the pattern block on `stream`.  With BMX_IGNORE_CASE in
+ * variant, the folded pattern's tables and block; the following scans of this scanner are case-insensitive. */
 int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t variant, void *stream);
 
 /* Starts a new result: zeroes the running count.  Positions of later bmx_scanner_scan calls are

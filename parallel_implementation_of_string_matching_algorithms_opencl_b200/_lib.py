@@ -23,6 +23,7 @@ VARIANT_QGRAM = 1
 VARIANT_WINDOW = 2
 VARIANT_SHIFTAND = 3
 VARIANT_NAMES = {0: "auto", 1: "qgram", 2: "window", 3: "shiftand"}
+IGNORE_CASE = 0x100   # BMX_IGNORE_CASE: OR'ed into a variant, ASCII case-insensitive search
 
 # every symbol include/bmx.h declares (tests/test_host_logic.py checks the header against this list)
 EXPORTS = [
@@ -53,7 +54,9 @@ class BmxStats(ctypes.Structure):
 
     def as_dict(self) -> dict:
         d = {name: getattr(self, name) for name, _ in self._fields_}
-        d["variant"] = VARIANT_NAMES.get(d["variant"], str(d["variant"]))
+        v = d["variant"]
+        d["variant"] = VARIANT_NAMES.get(v & ~IGNORE_CASE, str(v))
+        d["ignore_case"] = bool(v & IGNORE_CASE)   # the case-folding kernels ran
         return d
 
 

@@ -156,14 +156,27 @@ int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t 
 {
     if (!s || !pat) return fail(BMX_E_BADARG, "bmx_scanner_set_pattern: NULL argument");
     if (int rc = check_pattern(m)) return rc;
-    if (variant < BMX_VARIANT_AUTO || variant > BMX_VARIANT_SHIFTAND)
+    const int32_t base = variant & ~BMX_IGNORE_CASE;
+    if (base < BMX_VARIANT_AUTO || base > BMX_VARIANT_SHIFTAND)
         return fail(BMX_E_BADARG, "unknown variant %d", variant);
     BMX_CUDA(cudaSetDevice(s->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
 
     const unsigned char *p = reinterpret_cast<const unsigned char *>(pat);
-    const Filter filter = choose_filter(variant, p, m);
-    if (s->d_block && s->m == m && s->filter == filter && memcmp(s->pat.data(), p, (size_t)m) == 0) {
+    // BMX_IGNORE_CASE: everything below works on the folded pattern.  A pattern without an ASCII letter is its own
+    // fold and matches the same positions either way: it runs the exact kernels.
+    std::vector<unsigned char> folded;
+    bool fold = false;
+    if (variant & BMX_IGNORE_CASE) {
+        folded.resize((size_t)m);
+        for (int32_t i = 0; i < m; ++i) {
+            folded[(size_t)i] = ascii_lower(p[i]);
+            fold = fold || (unsigned)((p[i] | 0x20u) - 'a') < 26u;   // an ASCII letter
+        }
+        p = folded.data();
+    }
+    const Filter filter = choose_filter(base, p, m);
+    if (s->d_block && s->m == m && s->filter == filter && s->fold == fold && memcmp(s->pat.data(), p, (size_t)m) == 0) {
         // same pattern as last time (a caller searching many texts for one pattern): tables and device block stand.
         // The upload was ordered on pat_stream only; any other stream waits for it (an event wait, no copy).
         if (st != s->pat_stream) BMX_CUDA(cudaStreamWaitEvent(st, s->ev_pat, 0));
@@ -172,6 +185,7 @@ int bmx_scanner_set_pattern(bmx_scanner *s, const char *pat, int32_t m, int32_t 
     s->m = m;
     s->m_halo = 0;
     s->filter = filter;
+    s->fold = fold;
     s->pat.assign(p, p + m);
 
     // Host image of the device block: tables once per pattern (BoyreMoore.cpp:153-190).
@@ -222,7 +236,7 @@ int bmx_scanner_begin(bmx_scanner *s, int64_t *d_pos_out, int64_t pos_cap, void 
     s->find_epoch = 0;
     s->timing_open = false;
     s->stats = bmx_stats{};
-    s->stats.variant = s->m > 0 ? filter_variant(s->filter) : BMX_VARIANT_AUTO;
+    s->stats.variant = s->m > 0 ? filter_variant(s->filter) | (s->fold ? BMX_IGNORE_CASE : 0) : BMX_VARIANT_AUTO;
     // no device work here: the first scan of the search treats the carried state as zero (ScanArgs::first_scan)
     (void)stream;
     return BMX_OK;
@@ -248,7 +262,7 @@ int bmx_scanner_scan(bmx_scanner *s, const void *d_text, int64_t n, int64_t pos_
     a.pos_cap = s->pos_cap;
 
     ScanLaunch launch{};
-    if (int rc = plan_scan(s->device, s->filter, s->m_halo ? s->m_halo : s->m, s->positions, &a, &launch)) return rc;
+    if (int rc = plan_scan(s->device, s->filter, s->fold, s->m_halo ? s->m_halo : s->m, s->positions, &a, &launch)) return rc;
 
     // scratch: two "zero halves" [tickets 16 B | scan count u64 + pad | block_sum u32 x blocks | seg_count u16 x segs |
     //          item_flag u8 x items], each zero whenever a scan starts on it, followed by

@@ -147,6 +147,7 @@ struct ScanArgs {
 // Launch description produced by plan_scan() and consumed by launch_scan().
 struct ScanLaunch {
     Filter filter;
+    bool fold;              // case-insensitive instance (BMX_IGNORE_CASE)
     int tile_bytes;
     int grid;
     size_t smem_bytes;
@@ -154,7 +155,7 @@ struct ScanLaunch {
 
 // Host entry points implemented in bmx_scan.cu.
 Filter choose_filter(int requested_variant, const unsigned char *pat, int32_t m);
-int plan_scan(int device, Filter filter, int32_t m, bool positions, ScanArgs *args, ScanLaunch *out);
+int plan_scan(int device, Filter filter, bool fold, int32_t m, bool positions, ScanArgs *args, ScanLaunch *out);
 int launch_scan(const ScanArgs &args, const ScanLaunch &launch, bool positions, void *stream);
 int launch_emit(const ScanArgs &args, void *stream);
 int launch_export_result(const unsigned long long *d_count, const int64_t *d_pos, int64_t pos_cap, void *d_dst, int64_t head,
@@ -185,6 +186,8 @@ inline uint32_t le_word(const unsigned char *p, int nbytes)
     for (int i = 0; i < nbytes && i < 4; ++i) w |= (uint32_t)p[i] << (8 * i);
     return w;
 }
+// BMX_IGNORE_CASE's fold: 'A'..'Z' -> 'a'..'z', every other byte value unchanged (Python's bytes.lower()).
+inline unsigned char ascii_lower(unsigned char c) { return (unsigned)(c - 'A') < 26u ? (unsigned char)(c | 0x20u) : c; }
 // Hash multiplier of a word that contributes `bytes` bytes to a gram: K << (32 - 8*bytes) drops the bytes beyond it.
 inline uint32_t gram_multiplier(uint32_t K, int bytes) { return bytes >= 4 ? K : (bytes == 0 ? 0u : (K << (32 - 8 * bytes))); }
 // An integer environment knob, read on every call (tests change them between calls).

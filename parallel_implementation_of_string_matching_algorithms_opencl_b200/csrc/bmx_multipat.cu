@@ -152,6 +152,7 @@ int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, in
     bmx_scanner *s = c.scanner;
     // the scanner leaves single-pattern mode: its cached pattern block no longer describes proto
     s->filter = kMulti;
+    s->fold = false;
     s->pat.clear();
     s->proto = ScanArgs{};
     s->proto.m = im.m_min;

@@ -105,6 +105,32 @@ __device__ __forceinline__ void bar_sync_consumers()
 {
     asm volatile("barrier.cta.sync 1, %0;" ::"r"(kConsumerThreads) : "memory");
 }
+// ASCII case fold of four bytes at once ('A'..'Z' -> 'a'..'z', every other byte value unchanged): for a byte b < 0x80,
+// t + 0x3F reaches bit 7 iff b >= 'A' and t + 0x25 iff b > 'Z'; t <= 0x7F, so no sum carries into the next byte.
+__device__ __forceinline__ uint32_t fold_word(uint32_t w)
+{
+    const uint32_t t = w & 0x7F7F7F7Fu;
+    const uint32_t u = (t + 0x3F3F3F3Fu) & ~(t + 0x25252525u) & ~w & 0x80808080u;
+    return w | (u >> 2);
+}
+// Case-insensitive scans fold a whole stage ([16 B pre | tile | halo]) in place, once, before any warp reads it, so
+// every reader of the stage (filters, coop_verify16, verify_candidates, dense_tile, Shift-And) sees folded text.
+// The stores are generic-proxy writes to memory the next TMA copy (async proxy) overwrites: each thread orders its
+// stores before that copy with a proxy fence, ahead of its warp's arrival on empty[s].
+__device__ __forceinline__ void fold_stage(uint8_t *stage, uint32_t bytes, int tid)
+{
+    uint4 *p = reinterpret_cast<uint4 *>(stage);
+#pragma unroll 4
+    for (uint32_t i = (uint32_t)tid; i < bytes / 16u; i += kConsumerThreads) {
+        uint4 v = p[i];
+        v.x = fold_word(v.x);
+        v.y = fold_word(v.y);
+        v.z = fold_word(v.z);
+        v.w = fold_word(v.w);
+        p[i] = v;
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
 // ---------------------------------------------------------------------------------------------
 // Shared-memory control block (the stages follow it, 128-byte aligned)
 // ---------------------------------------------------------------------------------------------
@@ -147,10 +173,14 @@ __device__ __forceinline__ uint32_t load_u32_unaligned(const uint8_t *base, int6
 // cand holds the candidates of ALL FOUR slabs of the lane's share of a segment (16 bits each, slab sl at bits 16 sl ..):
 // one call per segment instead of one per slab -- candidates of different slabs usually sit in different lanes, and
 // lanes of one call verify concurrently, so a segment with candidates in three slabs pays for one verification, not three.
+// FOLD (case-insensitive scans): the pattern and tables are folded, and so is a staged tile, but text read from global
+// memory (m > kHaloSmemMax) is the caller's: its bytes are folded as they are compared and looked up in bad[].
+template <bool FOLD>
 __device__ __noinline__ unsigned long long verify_candidates(unsigned long long cand, const uint8_t *vbase, int64_t p0, int32_t m,
                                                              const uint8_t *pat, const uint32_t *rpat, const int32_t *bad,
                                                              const int32_t *good, bool wordwise)
 {
+    auto tb = [](uint8_t c) -> uint8_t { return FOLD && (uint32_t)(c - 'A') < 26u ? (uint8_t)(c | 0x20u) : c; };
     unsigned long long hits = 0;
     while (cand) {
         const int b = __ffsll((long long)cand) - 1;
@@ -190,13 +220,13 @@ __device__ __noinline__ unsigned long long verify_candidates(unsigned long long 
             }
         }
         if (!differs)
-            while (k < m && t[m - 1 - k] == pat[m - 1 - k]) ++k;
+            while (k < m && tb(t[m - 1 - k]) == pat[m - 1 - k]) ++k;
         int32_t shift;
         if (k == m) {
             hits |= 1ull << b;
             shift = 1;
         } else {
-            int32_t d1 = bad[t[m - 1]] - k;
+            int32_t d1 = bad[tb(t[m - 1])] - k;
             d1 = d1 > 1 ? d1 : 1;
             shift = d1;
             if (k > 0) {
@@ -578,7 +608,7 @@ struct VerifyCtx {
 // a tile without the any-pass and the vote -- every lane builds its masks right away.  Kept out of
 // line so the common path of scan_kernel stays exactly the sparse filter loop.  Returns the hits
 // found (count-only mode adds them up) with bit 63 set while the text is still dense.
-template <Filter F, int TILE, bool POSITIONS>
+template <Filter F, int TILE, bool POSITIONS, bool FOLD>
 __device__ __forceinline__ unsigned long long dense_tile_body(const ScanArgs &A, const uint8_t *st, int64_t tile_v0,
                                                               VerifyCtx vc, int warp, int lane)
 {
@@ -604,7 +634,7 @@ __device__ __forceinline__ unsigned long long dense_tile_body(const ScanArgs &A,
         }
         cand_lanes += __popc(__ballot_sync(0xFFFFFFFFu, cand64 != 0));
         if (cand64 && !vc.exact_filter)
-            cand64 = verify_candidates(cand64, vc.vbase, seg_p0, A.m, vc.pat, vc.rpat, vc.bad, vc.good, A.verify_smem != 0);
+            cand64 = verify_candidates<FOLD>(cand64, vc.vbase, seg_p0, A.m, vc.pat, vc.rpat, vc.bad, vc.good, A.verify_smem != 0);
 #pragma unroll
         for (int sl = 0; sl < 4; ++sl) hm[sl] = (uint32_t)(cand64 >> (16 * sl)) & 0xFFFFu;
         const uint32_t seg_hits = __popcll(cand64);
@@ -622,13 +652,15 @@ __device__ __forceinline__ unsigned long long dense_tile_body(const ScanArgs &A,
 // out of line the kernel arguments are reached through a generic pointer (LD.E, a long-scoreboard stall per segment:
 // profiles/r02_ncu_scan_eng_is.txt), inline they are constant-bank operands ('is' on English prose count-only 4.52 ->
 // 4.86 TB/s, ' ' 5.25 -> 5.78).  m = 3 stays out of line: inlined, its SPARSE path lost 7 % (bytes256: 6.6 -> 5.95 TB/s).
-template <Filter F, int TILE, bool POSITIONS>
+template <Filter F, int TILE, bool POSITIONS, bool FOLD>
 __device__ __noinline__ unsigned long long dense_tile(const ScanArgs &A, const uint8_t *st, int64_t tile_v0, VerifyCtx vc, int warp, int lane)
 {
-    return dense_tile_body<F, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
+    return dense_tile_body<F, TILE, POSITIONS, FOLD>(A, st, tile_v0, vc, warp, lane);
 }
 
-template <Filter F, int TILE, bool POSITIONS>
+// FOLD: case-insensitive scan (BMX_IGNORE_CASE).  The pattern block is folded on the host; the kernel folds each
+// staged tile (fold_stage) and the bytes it verifies from global memory.
+template <Filter F, int TILE, bool POSITIONS, bool FOLD>
 __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant__ ScanArgs A)
 {
     constexpr int WARP_BYTES = TILE / kConsumerWarps;   // contiguous bytes owned by one warp
@@ -767,7 +799,11 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
     for (uint32_t s = 0u, ph = 0u;; s = (s + 1u == S) ? 0u : s + 1u, ph ^= (s == 0u) ? 1u : 0u) {
         mbar_wait(&ctl->full[s], ph);
         const int32_t tile_s = ctl->slot_tile[s];
-        if (tile_s < 0) break;
+        if (tile_s < 0) break;   // taken by every warp at once: each warp below reaches the fold's barrier
+        if constexpr (FOLD) {
+            fold_stage(stages + (size_t)s * A.stage_stride, A.stage_stride, tid);
+            bar_sync_consumers();
+        }
         const uint32_t tile = (uint32_t)tile_s;
         const uint8_t *st = stages + (size_t)s * A.stage_stride + kPre;  // st[0] = first byte of the tile
         const int64_t tile_v0 = (int64_t)tile * TILE;
@@ -781,8 +817,8 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
             if (dense_mode) {
                 const VerifyCtx vc{vbase, pat, rpat, bad, good, exact_filter, all_valid};
                 unsigned long long r;
-                if constexpr (F == kBytes1 || F == kBytes2) r = dense_tile_body<F, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
-                else r = dense_tile<F, TILE, POSITIONS>(A, st, tile_v0, vc, warp, lane);
+                if constexpr (F == kBytes1 || F == kBytes2) r = dense_tile_body<F, TILE, POSITIONS, FOLD>(A, st, tile_v0, vc, warp, lane);
+                else r = dense_tile<F, TILE, POSITIONS, FOLD>(A, st, tile_v0, vc, warp, lane);
                 dense_mode = (r >> 63) != 0;
                 if (!POSITIONS) my_count += r & ~(1ull << 63);
                 took_dense = true;
@@ -851,7 +887,7 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
                                     uint32_t cand = filter_mask<F>(w[sl], w4[sl], A);
                                     if (!all_valid) cand &= valid_bits(p0, A.vmin, A.vmax);
                                     if (cand)
-                                        hm[sl] = exact_filter ? cand : (uint32_t)verify_candidates(cand, vbase, p0, A.m, pat, rpat, bad, good, A.verify_smem != 0);
+                                        hm[sl] = exact_filter ? cand : (uint32_t)verify_candidates<FOLD>(cand, vbase, p0, A.m, pat, rpat, bad, good, A.verify_smem != 0);
                                     seg_hits += __popc(hm[sl]);
                                 }
                             }
@@ -1438,23 +1474,34 @@ void fill_filter_constants(Filter filter, const unsigned char *pat, int32_t m, S
     }
 }
 
-// The scan_kernel instances of one filter kind: [tile is 32 KiB][positions mode].
+// The scan_kernel instances of one filter kind: [case-folding][tile is 32 KiB][positions mode].  The multi-pattern kind
+// has no folding instances (nullptr).
 struct KernelRow {
-    const void *k[2][2];
+    const void *k[2][2][2];
 };
+template <Filter F, bool FOLD>
+static void fill_row(const void *(&k)[2][2])
+{
+    k[0][0] = (const void *)&scan_kernel<F, 16384, false, FOLD>;
+    k[0][1] = (const void *)&scan_kernel<F, 16384, true, FOLD>;
+    k[1][0] = (const void *)&scan_kernel<F, 32768, false, FOLD>;
+    k[1][1] = (const void *)&scan_kernel<F, 32768, true, FOLD>;
+}
 template <Filter F>
 static KernelRow kernels_of()
 {
-    return {{{(const void *)&scan_kernel<F, 16384, false>, (const void *)&scan_kernel<F, 16384, true>},
-             {(const void *)&scan_kernel<F, 32768, false>, (const void *)&scan_kernel<F, 32768, true>}}};
+    KernelRow r{};
+    fill_row<F, false>(r.k[0]);
+    if constexpr (F != kMulti) fill_row<F, true>(r.k[1]);
+    return r;
 }
-static const void *scan_kernel_for(Filter filter, int tile, bool positions)
+static const void *scan_kernel_for(Filter filter, int tile, bool positions, bool fold)
 {
     static const KernelRow rows[] = {kernels_of<kQgramPerResidue>(), kernels_of<kQgram>(), kernels_of<kWindow4>(),
                                      kernels_of<kBytes1>(),          kernels_of<kBytes2>(), kernels_of<kBytes3>(),
                                      kernels_of<kBytes5>(),          kernels_of<kShiftAnd>(), kernels_of<kMulti>()};
     static_assert(sizeof rows / sizeof rows[0] == kFilterCount, "one row per filter kind, in the order of enum Filter");
-    return rows[filter].k[tile == 32768][positions];
+    return rows[filter].k[fold][tile == 32768][positions];
 }
 
 // Device attributes (and the expand kernel's occupancy) are queried once per device, under a mutex: a search on
@@ -1490,7 +1537,7 @@ static int device_info(int device, int *sm_count, int *smem_optin, int *smem_sm,
     return BMX_OK;
 }
 
-int plan_scan(int device, Filter filter, int32_t m, bool positions, ScanArgs *a, ScanLaunch *out)
+int plan_scan(int device, Filter filter, bool fold, int32_t m, bool positions, ScanArgs *a, ScanLaunch *out)
 {
     int sm_count = 0, smem_optin = 0, smem_sm = 0;
     if (int rc = device_info(device, &sm_count, &smem_optin, &smem_sm, nullptr)) return rc;
@@ -1524,6 +1571,7 @@ int plan_scan(int device, Filter filter, int32_t m, bool positions, ScanArgs *a,
     a->stages = (uint32_t)stages;
 
     out->filter = filter;
+    out->fold = fold;
     out->tile_bytes = tile;
     out->smem_bytes = kCtlBytes + a->multi_smem + (size_t)stages * a->stage_stride;
     const int64_t tiles = (a->vlen + tile - 1) / tile;
@@ -1541,7 +1589,7 @@ int plan_scan(int device, Filter filter, int32_t m, bool positions, ScanArgs *a,
     const int spare = std::max(0, std::min(sm_count - 1, env_int("BMX_SPARE_SMS", 0)));
     out->grid = (int)std::min<int64_t>(tiles, (int64_t)(sm_count - spare) * ctas_per_sm);
 
-    const void *k = scan_kernel_for(filter, tile, positions);
+    const void *k = scan_kernel_for(filter, tile, positions, fold);
     {
         // the opt-in shared-memory limit of a kernel is raised once per (device, kernel, size)
         static std::map<std::pair<int, const void *>, size_t> granted;
@@ -1559,7 +1607,7 @@ int plan_scan(int device, Filter filter, int32_t m, bool positions, ScanArgs *a,
 
 int launch_scan(const ScanArgs &a, const ScanLaunch &l, bool positions, void *stream)
 {
-    const void *k = scan_kernel_for(l.filter, l.tile_bytes, positions);
+    const void *k = scan_kernel_for(l.filter, l.tile_bytes, positions, l.fold);
     void *params[] = {const_cast<ScanArgs *>(&a)};
     const cudaError_t e = cudaLaunchKernel(k, dim3((unsigned)l.grid), dim3(kThreads), params, l.smem_bytes,
                                            static_cast<cudaStream_t>(stream));

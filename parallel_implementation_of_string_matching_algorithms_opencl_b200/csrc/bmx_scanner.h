@@ -14,6 +14,7 @@ struct bmx_scanner {
     int32_t m = 0;             // pattern length (multi-pattern mode: the shortest one -- it bounds the start positions of a scan)
     int32_t m_halo = 0;        // multi-pattern mode: the longest pattern (sizes the staged halo); 0 = m
     bmx::Filter filter = bmx::kQgram;   // the scan kernel's filter kind (kMulti in multi-pattern mode)
+    bool fold = false;         // case-insensitive scans (BMX_IGNORE_CASE with a pattern that has an ASCII letter): pat is folded
     cudaEvent_t ev_pat = nullptr; // recorded behind the upload of the block
     cudaStream_t pat_stream = nullptr;
     std::vector<unsigned char> pat;

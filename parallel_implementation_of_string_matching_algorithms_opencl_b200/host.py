@@ -28,10 +28,11 @@ from ._lib import BmxStats, check
 _VARIANTS = {"auto": 0, "qgram": 1, "window": 2, "shiftand": 3}
 
 
-def _variant(v) -> int:
+def _variant(v, ignore_case: bool = False) -> int:
+    flag = _lib.IGNORE_CASE if ignore_case else 0
     if isinstance(v, str):
-        return _VARIANTS[v]
-    return int(v)
+        return _VARIANTS[v] | flag
+    return int(v) | flag
 
 
 def _as_bytes(pattern) -> bytes:
@@ -86,11 +87,12 @@ def _host_text(text):
 
 
 def search(text, pattern, max_positions: int | None = None, variant="auto", device: int | None = None,
-           return_stats: bool = False):
+           return_stats: bool = False, ignore_case: bool = False):
     """Serial-reference result for host text: (count, positions[int64]) -- BoyreMoore.cpp:192-313.
 
     positions holds min(count, max_positions) ascending start offsets (default: room for all).
-    max_positions=0 is count-only.
+    max_positions=0 is count-only.  ignore_case=True matches ASCII letters in either case (BMX_IGNORE_CASE):
+    the result for text.lower() and pattern.lower(), without touching the text.
     """
     lib = _lib.load()
     pat = _as_bytes(pattern)
@@ -107,7 +109,7 @@ def search(text, pattern, max_positions: int | None = None, variant="auto", devi
     while True:
         pos = np.empty(cap, dtype=np.int64)
         check(lib.bmx_search_ex(device, ptr, n, pat, len(pat), pos.ctypes.data if cap else None,
-                                cap, ctypes.byref(count), _variant(variant), ctypes.byref(stats)))
+                                cap, ctypes.byref(count), _variant(variant, ignore_case), ctypes.byref(stats)))
         if not open_ended or count.value <= cap:
             break
         cap = int(count.value)
@@ -121,13 +123,14 @@ def _first_cap(n: int, m: int) -> int:
 
 
 def search_device(text, pattern, pos_out=None, max_positions: int | None = None, pos_base: int = 0,
-                  variant="auto", stream=None, timing: bool = True):
+                  variant="auto", stream=None, timing: bool = True, ignore_case: bool = False):
     """Scan a CUDA uint8 tensor -- BoyreMoore.cpp:258-286.  Returns (count, positions, stats).
 
     pos_out: optional preallocated int64 CUDA tensor; otherwise max_positions (default 0 =
     count-only) entries are allocated.  positions is the filled prefix of that tensor (or None).
     Every reported position has pos_base added (multi-GPU shards report global offsets).
     timing=False skips the library's CUDA-event instrumentation (a few microseconds per call): stats is then {}.
+    ignore_case=True: ASCII case-insensitive, as search(); the tensor is left as it was.
     """
     import torch
 
@@ -147,7 +150,8 @@ def search_device(text, pattern, pos_out=None, max_positions: int | None = None,
         stats = BmxStats()
         check(lib.bmx_search_device_ex(c_void_p(text.data_ptr() if n else 0), n, pat, len(pat), c_int64(pos_base),
                                        c_void_p(pos_out.data_ptr()) if cap else None, cap, ctypes.byref(count),
-                                       _variant(variant), ctypes.byref(stats) if timing else None, c_void_p(s.cuda_stream)))
+                                       _variant(variant, ignore_case), ctypes.byref(stats) if timing else None,
+                                       c_void_p(s.cuda_stream)))
     found = None if pos_out is None else pos_out[: min(count.value, cap)]
     return count.value, found, (stats.as_dict() if timing else {})
 
@@ -347,9 +351,10 @@ class Scanner:
         except Exception:
             pass
 
-    def set_pattern(self, pattern, variant="auto", stream=0):
+    def set_pattern(self, pattern, variant="auto", stream=0, ignore_case: bool = False):
+        """ignore_case=True: the following scans match ASCII letters in either case (BMX_IGNORE_CASE)."""
         pat = _as_bytes(pattern)
-        check(self._lib.bmx_scanner_set_pattern(self._h, pat, len(pat), _variant(variant), c_void_p(stream)))
+        check(self._lib.bmx_scanner_set_pattern(self._h, pat, len(pat), _variant(variant, ignore_case), c_void_p(stream)))
 
     def begin(self, pos_out=None, stream=0):
         cap = 0 if pos_out is None else pos_out.numel()

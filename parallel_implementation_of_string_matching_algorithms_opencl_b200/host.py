@@ -332,6 +332,14 @@ def search_ranges_device(text, pattern, begin, end, max_positions: int = 0, stre
     return counts, offsets, None if pos is None else pos[: min(total.value, cap)]
 
 
+def _check_cuda(t, dtype: str, what: str):
+    """The scanner takes raw device pointers: a CPU, strided or wrongly typed tensor would be read as other bytes."""
+    import torch
+
+    if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype != getattr(torch, dtype) or not t.is_contiguous():
+        raise TypeError(f"{what} must be a contiguous CUDA {dtype} tensor")
+
+
 class Scanner:
     """Reusable scanner (bmx_scanner_*): pattern block + look-back scratch kept across scans."""
 
@@ -357,10 +365,13 @@ class Scanner:
         check(self._lib.bmx_scanner_set_pattern(self._h, pat, len(pat), _variant(variant, ignore_case), c_void_p(stream)))
 
     def begin(self, pos_out=None, stream=0):
+        if pos_out is not None:
+            _check_cuda(pos_out, "int64", "Scanner.begin(): pos_out")
         cap = 0 if pos_out is None else pos_out.numel()
         check(self._lib.bmx_scanner_begin(self._h, c_void_p(pos_out.data_ptr()) if cap else None, cap, c_void_p(stream)))
 
     def scan(self, text, pos_base=0, stream=0):
+        _check_cuda(text, "uint8", "Scanner.scan(): text")
         check(self._lib.bmx_scanner_scan(self._h, c_void_p(text.data_ptr()), text.numel(), c_int64(pos_base), c_void_p(stream)))
 
     def set_timing(self, level: int):
@@ -370,6 +381,7 @@ class Scanner:
     def export_result(self, packed, stream=0):
         """Enqueue {count, positions written, first len(packed)-2 positions} into the int64 CUDA
         tensor `packed` (no host sync): the send buffer of the multi-GPU exchange step."""
+        _check_cuda(packed, "int64", "Scanner.export_result(): packed")
         check(self._lib.bmx_scanner_export_result(self._h, c_void_p(packed.data_ptr()), packed.numel() - 2, c_void_p(stream)))
 
     def finish(self, stream=0):

@@ -224,6 +224,33 @@ int bmx_search_ranges_device(const void *d_text, int64_t n, int64_t nranges,
                              uint64_t *total_out, void *stream);
 
 /*
+ * Dictionary search (grep -F -f wordlist): up to 65536 fixed strings in ONE pass over the text, matches reported in
+ * text order as (position, pattern) pairs.  bmx_dict_create hashes the set once into a device block the handle owns
+ * (the candidate table of bmx_search_multi, sized by the set: DESIGN §3.11); every search reuses it.
+ *   create     1 <= npat <= 65536 patterns, each 7 <= ms[k] <= 4096 bytes (BMX_E_BADARG otherwise, naming the
+ *              first bad one).  The handle lives on `device`, is immutable after create and may be used from
+ *              several host threads at once, each with its own stream; scratch comes from the calling thread's
+ *              context, as for every other entry point.
+ *   result     a match is a pair (p, k) with text[p..p+ms[k]) == pats[k]; overlapping matches count.  The list of
+ *              all pairs is sorted by p, then by k (patterns sharing a prefix, and duplicate patterns, tie at one p:
+ *              every duplicate is reported).  counts[k] (host, npat entries) = pairs of pattern k, always exact;
+ *              *total_out = their sum.  pos_out[i], pat_out[i] for i < min(total, cap) are exactly the first
+ *              min(total, cap) pairs, positions with pos_base added.  The pairs of pattern k are what bmx_search_ex
+ *              returns for that pattern alone (and, for npat <= 64, what bmx_search_multi returns for k).
+ * bmx_dict_search_device: d_text, d_pos_out, d_pat_out are DEVICE memory on the dictionary's device (both outputs
+ * NULL: counts only); synchronous on `stream`.  bmx_dict_search: host text, copied to the device once (a text that
+ * does not fit there is BMX_E_NOMEM); outputs in host memory.
+ */
+typedef struct bmx_dict bmx_dict;
+int bmx_dict_create(int device, int32_t npat, const char *const *pats, const int32_t *ms, bmx_dict **out);
+void bmx_dict_destroy(bmx_dict *d);
+int bmx_dict_search_device(const bmx_dict *d, const void *d_text, int64_t n, int64_t pos_base,
+                           int64_t *d_pos_out, int32_t *d_pat_out, int64_t cap,
+                           uint64_t *counts, uint64_t *total_out, void *stream);
+int bmx_dict_search(const bmx_dict *d, const char *text, int64_t n,
+                    int64_t *pos_out, int32_t *pat_out, int64_t cap, uint64_t *counts, uint64_t *total_out);
+
+/*
  * The reference's host-side word partitioner -- replaces BoyreMoore.cpp:94-141.  Splits
  * text[0..n) (up to the first NUL, like the reference's strcpy'd copy, :89-90) on single spaces
  * into nparts inclusive byte ranges of equal word count: se[2*p], se[2*p+1].  The space between

@@ -35,6 +35,7 @@ EXPORTS = [
     "bmx_mg_search_device", "bmx_exchange_create", "bmx_exchange_destroy", "bmx_exchange_handle", "bmx_exchange_connect",
     "bmx_exchange_connect_local", "bmx_exchange_post", "bmx_exchange_collect", "bmx_exchange_wait", "bmx_release_memory", "bmx_search_multi_device",
     "bmx_search_ranges", "bmx_search_ranges_device",
+    "bmx_dict_create", "bmx_dict_destroy", "bmx_dict_search", "bmx_dict_search_device",
 ]
 
 
@@ -103,6 +104,12 @@ def load() -> ctypes.CDLL:
                                       c_void_p, c_int64, c_void_p, c_void_p]
     lib.bmx_search_ranges_device.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_char_p, c_int32,
                                              c_void_p, c_int64, c_void_p, c_void_p, POINTER(c_uint64), c_void_p]
+    lib.bmx_dict_create.argtypes = [c_int, c_int32, POINTER(c_char_p), POINTER(c_int32), POINTER(c_void_p)]
+    lib.bmx_dict_destroy.argtypes = [c_void_p]
+    lib.bmx_dict_destroy.restype = None
+    lib.bmx_dict_search.argtypes = [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p, POINTER(c_uint64)]
+    lib.bmx_dict_search_device.argtypes = [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                           POINTER(c_uint64), c_void_p]
     lib.bmx_scanner_create.argtypes = [c_int, POINTER(c_void_p)]
     lib.bmx_scanner_destroy.argtypes = [c_void_p]
     lib.bmx_scanner_destroy.restype = None

@@ -15,7 +15,7 @@ CSRC = PKG_DIR / "csrc"
 LIB_PATH = PKG_DIR / "libbmx.so"
 REFMAIN_PATH = PKG_DIR / "bmx_refmain"
 
-SOURCES = ["bmx_scan.cu", "bmx_abi.cu", "bmx_host.cu", "bmx_multi.cu", "bmx_multipat.cu", "bmx_exchange.cu", "bmx_ranges.cu", "bmx_tables.cpp", "bmx_partition.cpp"]
+SOURCES = ["bmx_scan.cu", "bmx_abi.cu", "bmx_host.cu", "bmx_multi.cu", "bmx_multipat.cu", "bmx_exchange.cu", "bmx_ranges.cu", "bmx_dict.cu", "bmx_tables.cpp", "bmx_partition.cpp"]
 HEADERS = ["bmx_internal.h", "bmx_scanner.h", "bmx_ctx.h", "../../include/bmx.h"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17",

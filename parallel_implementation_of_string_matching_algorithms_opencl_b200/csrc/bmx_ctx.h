@@ -88,6 +88,8 @@ inline int64_t first_pos_room(const ThreadCtx &c, int64_t n, int32_t m, int64_t 
 // One shard of a host text through the calling GPU's context (bmx_host.cu, used by bmx_multi.cu).
 int ingest_shard(ThreadCtx &ctx, int device, const char *text, int64_t n, const char *pat, int32_t m, int64_t pos_base,
                  int64_t want_cap, uint64_t *count, int64_t *dev_cap);
+// A host text copied once into ctx.text (the chunked ingest without a scan); NOMEM when it does not fit (bmx_host.cu).
+int copy_text_resident(ThreadCtx &ctx, const char *text, int64_t n);
 
 // Per-range counts, offsets and positions of host ranges over a host text (bmx_ranges.cu).  The ranges are checked
 // (inside [0, n], begin <= end) and cover [lo, hi); counts / offsets / pos_out are host memory.
@@ -99,6 +101,58 @@ int search_ranges_host(ThreadCtx &c, const char *text, int64_t n, int64_t nrange
 bool multi_eligible(int32_t npat, const int32_t *ms);
 int multi_scan_resident(ThreadCtx &c, const unsigned char *d_text, int64_t n, int32_t npat, const char *const *pats,
                         const int32_t *ms, int64_t *const *d_out, const int64_t *caps, uint64_t *counts, cudaStream_t st);
+
+// The shared candidate table of a pattern set (bmx_multipat.cu; used by bmx_search_multi and the dictionaries).  One
+// gram length q = min(12, m_min - 3) = 4 + q2 + q3 bytes for every pattern and residue.
+struct SetHash {
+    int32_t m_min = 0, m_max = 0;
+    int q2 = 0, q3 = 0;              // bytes the second and third word contribute to a gram
+    uint32_t hmul = 0, hmul2 = 0;    // their multipliers (gram_multiplier: the bytes beyond the gram drop out)
+};
+SetHash set_hash(int32_t npat, const int32_t *ms);
+// Hash of the gram that starts at p (host and device alike: the scan hashes aligned text words the same way).
+__host__ __device__ inline uint32_t set_gram_hash(const SetHash &sh, const unsigned char *p)
+{
+    uint32_t w0 = 0u, w1 = 0u, w2 = 0u;
+    for (int i = 0; i < 4; ++i) w0 |= (uint32_t)p[i] << (8 * i);
+    for (int i = 0; i < sh.q2; ++i) w1 |= (uint32_t)p[4 + i] << (8 * i);
+    for (int i = 0; i < sh.q3; ++i) w2 |= (uint32_t)p[8 + i] << (8 * i);
+    return w0 + sh.hmul * w1 + sh.hmul2 * w2;
+}
+// Bytes of the pattern blob: every pattern 16-byte aligned and followed by at least 8 bytes of padding.
+size_t set_blob_bytes(int32_t npat, const int32_t *ms);
+// Fills bitmap (kMultiBitmapWords words), exact table (2^slots_log2 slots, load <= 1/2), directory and blob, all zeroed
+// by the caller: table entry {hash, 0x80000000 | k << 2 | r} for the gram P_k[r .. r+q) of every pattern k and residue r.
+void fill_set_tables(int32_t npat, const char *const *pats, const int32_t *ms, const SetHash &sh, int slots_log2, uint32_t *bits,
+                     uint2 *table, uint2 *dir, unsigned char *blob);
+
+#ifdef __CUDACC__
+// Exclusive prefix of v over a CTA of THREADS threads; *total receives the CTA's sum.  Every thread calls it.
+template <int THREADS>
+__device__ __forceinline__ unsigned long long cta_exclusive_scan(unsigned long long v, unsigned long long *total)
+{
+    __shared__ unsigned long long warp_total[THREADS / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned long long x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned long long y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= o) x += y;
+    }
+    if (lane == 31) warp_total[warp] = x;
+    __syncthreads();
+    unsigned long long base = 0, sum = 0;
+#pragma unroll
+    for (int w = 0; w < THREADS / 32; ++w) {
+        const unsigned long long t = warp_total[w];
+        base += w < warp ? t : 0ull;
+        sum += t;
+    }
+    __syncthreads();   // warp_total may be reused by the next call
+    *total = sum;
+    return base + x - v;
+}
+#endif
 
 // Sets the scanner's timing level (bmx_scanner_set_timing) for the scope and restores the caller's level after it.
 class ScopedTiming {

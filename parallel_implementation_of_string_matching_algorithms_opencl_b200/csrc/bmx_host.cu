@@ -323,6 +323,13 @@ int ingest_shard(ThreadCtx &ctx, int device, const char *text, int64_t n, const 
     *dev_cap = io.dev_cap;
     return rc;
 }
+
+int copy_text_resident(ThreadCtx &ctx, const char *text, int64_t n)
+{
+    Ingest io;
+    io.copy_only = true;
+    return ingest_and_scan(ctx, ctx.device, text, n, "", 1, 0, BMX_VARIANT_AUTO, &io);   // (a copy reads no pattern)
+}
 }  // namespace bmx
 
 extern "C" {

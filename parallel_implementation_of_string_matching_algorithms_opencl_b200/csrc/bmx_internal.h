@@ -54,10 +54,13 @@ enum Filter : int {
     kBytes5,            // WINDOW, m = 5, 6 on small alphabets: the first five bytes, four start positions per word
     kShiftAnd,          // SHIFTAND, m <= 32
     kMulti,             // a multi-pattern set (bmx_multipat.cu)
+    kDict,              // a dictionary (bmx_dict.cu): kMulti's filter with the table geometry set per dictionary
     kFilterCount
 };
 
-// The public bmx_variant a kind belongs to (kMulti belongs to none: AUTO).
+// Kinds that scan for a pattern set through the shared candidate table.
+constexpr __host__ __device__ bool filter_is_set(Filter f) { return f == kMulti || f == kDict; }
+// The public bmx_variant a kind belongs to (the set kinds belong to none: AUTO).
 constexpr __host__ __device__ int filter_variant(Filter f)
 {
     if (f == kQgramPerResidue || f == kQgram) return BMX_VARIANT_QGRAM;
@@ -65,7 +68,7 @@ constexpr __host__ __device__ int filter_variant(Filter f)
     return f == kShiftAnd ? BMX_VARIANT_SHIFTAND : BMX_VARIANT_AUTO;
 }
 // Start position of mask bit 0 relative to its 16-byte chunk: the q-gram hashes flag starts up to 3 bytes in front.
-constexpr __host__ __device__ int filter_owner_offset(Filter f) { return f == kQgramPerResidue || f == kQgram || f == kMulti ? -3 : 0; }
+constexpr __host__ __device__ int filter_owner_offset(Filter f) { return f == kQgramPerResidue || f == kQgram || filter_is_set(f) ? -3 : 0; }
 // Pattern bytes a byte-parallel kind tests (0: not byte-parallel).
 constexpr __host__ __device__ int filter_bytes(Filter f)
 {
@@ -142,6 +145,10 @@ struct ScanArgs {
     uint32_t first_scan;                   // first scan of a search: carry_in / count_acc count as 0 (no memset needed)
     void *zero_ptr;                        // expand kernel: the OTHER zero-initialised scratch half, left dirty by the scan before
     uint32_t zero_vec16;                   //   this one; its first zero_vec16 16-byte words are cleared for the next scan (0: nothing)
+    // dictionary variant (kDict; last, so that no field in front of them moves): the dictionary's table geometry
+    uint32_t mslots_log2;                  // the exact table has 2^mslots_log2 slots
+    uint32_t mtable_smem;                  // 1: the exact table is staged into shared memory, 0: read from global memory (L2)
+    uint32_t mocc_log2;                    // bits of the staged "home slot occupied" array: bit (slot & (2^mocc_log2 - 1))
 };
 
 // Launch description produced by plan_scan() and consumed by launch_scan().
@@ -176,6 +183,16 @@ constexpr int kMultiSlots = 1 << kMultiSlotsLog2;
 constexpr uint32_t kMultiSlotMul = 0x85EBCA6Bu;
 constexpr uint32_t kHashMul2 = 0xC2B2AE3Du;
 constexpr size_t kMultiSmemBytes = (size_t)kMultiBitmapWords * 4 + (size_t)kMultiSlots * 8 + (size_t)kMultiMaxPatterns * 8;
+// dictionaries (bmx_dict.cu): table of the next power of two >= 8 K slots (load <= 1/2), at least kMultiSlots
+constexpr int kDictMaxPatterns = 65536;
+constexpr int kDictMaxOccLog2 = 15;          // the occupancy array is folded to at most 2^15 bits = 4 KiB
+constexpr int kDictMaxSmemSlotsLog2 = 11;    // tables of up to 2^11 slots (16 KiB, K <= 256) are staged into shared memory
+// Shared memory a kDict scan keeps in front of its stages: bitmap | occupancy bits | (table, when staged).
+constexpr __host__ __device__ size_t dict_smem_bytes(uint32_t slots_log2, uint32_t table_smem, uint32_t occ_log2)
+{
+    return (((size_t)kMultiBitmapWords * 4 + ((size_t)1 << occ_log2) / 8 + (table_smem ? ((size_t)8 << slots_log2) : 0)) + 127) &
+           ~size_t(127);
+}
 constexpr unsigned long long kFindMask = (1ull << 47) - 1;   // find-first keys: positions below 2^47
 
 // ---- host helpers -------------------------------------------------------------------------

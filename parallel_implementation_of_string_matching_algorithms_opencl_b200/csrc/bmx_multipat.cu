@@ -42,14 +42,11 @@ struct MultiImage {
 
 void build_multi_image(int32_t npat, const char *const *pats, const int32_t *ms, MultiImage *im)
 {
-    im->m_min = *std::min_element(ms, ms + npat);
-    im->m_max = *std::max_element(ms, ms + npat);
-    // one gram length for all patterns and residues: q = min(12, m_min - 3) bytes = 4 + q2 (second word) + q3 (third word)
-    const int q = std::min(12, im->m_min - 3);
-    const int q2 = std::min(4, q - 4), q3 = std::max(0, q - 8);
-    im->hmul = gram_multiplier(kHashMul, q2);
-    im->hmul2 = gram_multiplier(kHashMul2, q3);
-    auto align16 = [](size_t v) { return (v + 15) & ~size_t(15); };
+    const SetHash sh = set_hash(npat, ms);
+    im->m_min = sh.m_min;
+    im->m_max = sh.m_max;
+    im->hmul = sh.hmul;
+    im->hmul2 = sh.hmul2;
     im->off_table = (size_t)kMultiBitmapWords * 4;
     im->off_dir = im->off_table + (size_t)kMultiSlots * 8;
     im->off_counts = im->off_dir + (size_t)kMultiMaxPatterns * 8;
@@ -57,27 +54,10 @@ void build_multi_image(int32_t npat, const char *const *pats, const int32_t *ms,
     im->off_out = im->off_split + (size_t)kMultiMaxPatterns * 8;
     im->off_caps = im->off_out + (size_t)kMultiMaxPatterns * 8;
     im->off_blob = im->off_caps + (size_t)kMultiMaxPatterns * 8;
-    size_t blob = 0;
-    for (int32_t k = 0; k < npat; ++k) blob += align16((size_t)ms[k] + 8);
-    im->bytes.assign(im->off_blob + blob + 16, 0);
-    uint32_t *bits = reinterpret_cast<uint32_t *>(im->bytes.data());
-    uint2 *table = reinterpret_cast<uint2 *>(im->bytes.data() + im->off_table);
-    uint2 *dir = reinterpret_cast<uint2 *>(im->bytes.data() + im->off_dir);
-    size_t at = 0;
-    for (int32_t k = 0; k < npat; ++k) {
-        const unsigned char *p = reinterpret_cast<const unsigned char *>(pats[k]);
-        memcpy(im->bytes.data() + im->off_blob + at, p, (size_t)ms[k]);
-        dir[k] = make_uint2((uint32_t)at, (uint32_t)ms[k]);
-        at += align16((size_t)ms[k] + 8);
-        for (int r = 0; r < 4; ++r) {   // pattern byte r on a word boundary: the gram P[r .. r+q)
-            const uint32_t h = le_word(p + r, 4) + im->hmul * le_word(p + r + 4, q2) + im->hmul2 * le_word(p + r + 8, q3);
-            const uint32_t b = h >> (32 - kMultiBitmapLog2);
-            bits[b >> 5] |= 1u << (b & 31u);
-            uint32_t slot = (h * kMultiSlotMul) >> (32 - kMultiSlotsLog2);
-            while (table[slot].y != 0u) slot = (slot + 1) & (kMultiSlots - 1);
-            table[slot] = make_uint2(h, 0x80000000u | ((uint32_t)k << 2) | (uint32_t)r);
-        }
-    }
+    im->bytes.assign(im->off_blob + set_blob_bytes(npat, ms) + 16, 0);
+    fill_set_tables(npat, pats, ms, sh, kMultiSlotsLog2, reinterpret_cast<uint32_t *>(im->bytes.data()),
+                    reinterpret_cast<uint2 *>(im->bytes.data() + im->off_table), reinterpret_cast<uint2 *>(im->bytes.data() + im->off_dir),
+                    im->bytes.data() + im->off_blob);
 }
 
 // One CTA per pattern: the starts of U at which pattern k matches, at their ranks.
@@ -126,6 +106,48 @@ __global__ void __launch_bounds__(kSplitThreads) multi_split_kernel(const int64_
 }  // namespace
 
 namespace bmx {
+
+SetHash set_hash(int32_t npat, const int32_t *ms)
+{
+    SetHash sh;
+    sh.m_min = *std::min_element(ms, ms + npat);
+    sh.m_max = *std::max_element(ms, ms + npat);
+    // one gram length for all patterns and residues: q = min(12, m_min - 3) bytes = 4 + q2 (second word) + q3 (third word)
+    const int q = std::min(12, sh.m_min - 3);
+    sh.q2 = std::min(4, q - 4);
+    sh.q3 = std::max(0, q - 8);
+    sh.hmul = gram_multiplier(kHashMul, sh.q2);
+    sh.hmul2 = gram_multiplier(kHashMul2, sh.q3);
+    return sh;
+}
+
+size_t set_blob_bytes(int32_t npat, const int32_t *ms)
+{
+    size_t blob = 0;
+    for (int32_t k = 0; k < npat; ++k) blob += ((size_t)ms[k] + 8 + 15) & ~size_t(15);
+    return blob;
+}
+
+void fill_set_tables(int32_t npat, const char *const *pats, const int32_t *ms, const SetHash &sh, int slots_log2, uint32_t *bits,
+                     uint2 *table, uint2 *dir, unsigned char *blob)
+{
+    const uint32_t mask = (1u << slots_log2) - 1u;
+    size_t at = 0;
+    for (int32_t k = 0; k < npat; ++k) {
+        const unsigned char *p = reinterpret_cast<const unsigned char *>(pats[k]);
+        memcpy(blob + at, p, (size_t)ms[k]);
+        dir[k] = make_uint2((uint32_t)at, (uint32_t)ms[k]);
+        at += ((size_t)ms[k] + 8 + 15) & ~size_t(15);
+        for (int r = 0; r < 4; ++r) {   // pattern byte r on a word boundary: the gram P[r .. r+q)
+            const uint32_t h = set_gram_hash(sh, p + r);
+            const uint32_t b = h >> (32 - kMultiBitmapLog2);
+            bits[b >> 5] |= 1u << (b & 31u);
+            uint32_t slot = (h * kMultiSlotMul) >> (32 - slots_log2);
+            while (table[slot].y != 0u) slot = (slot + 1) & mask;
+            table[slot] = make_uint2(h, 0x80000000u | ((uint32_t)k << 2) | (uint32_t)r);
+        }
+    }
+}
 
 // All K patterns over device-resident text d_text[0..n) in one pass (eligible sets only).  d_out[k] (device buffer of
 // caps[k] entries, or NULL) receives pattern k's first min(counts[k], caps[k]) starts, ascending; counts[k] is exact.

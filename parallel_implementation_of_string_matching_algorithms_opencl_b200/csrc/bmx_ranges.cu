@@ -59,31 +59,6 @@ __device__ __forceinline__ int64_t upper_bound(const int64_t *a, int64_t lo, int
     return lo;
 }
 
-// Exclusive prefix of v over the CTA (kRangeThreads threads); *total receives the CTA's sum.
-__device__ __forceinline__ unsigned long long cta_exclusive_scan(unsigned long long v, unsigned long long *total)
-{
-    __shared__ unsigned long long warp_total[kRangeThreads / 32];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned long long x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const unsigned long long y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_total[warp] = x;
-    __syncthreads();
-    unsigned long long base = 0, sum = 0;
-#pragma unroll
-    for (int w = 0; w < kRangeThreads / 32; ++w) {
-        const unsigned long long t = warp_total[w];
-        base += w < warp ? t : 0ull;
-        sum += t;
-    }
-    __syncthreads();   // warp_total may be reused by the next call
-    *total = sum;
-    return base + x - v;
-}
-
 // Entries of L the scan left: min(count, cap) when the count is on the device, else `cap` itself.
 __device__ __forceinline__ int64_t held_entries(const unsigned long long *d_count, int64_t cap)
 {
@@ -114,7 +89,7 @@ __global__ void __launch_bounds__(kRangeThreads) range_rank_kernel(
         sum += (unsigned long long)c;
     }
     unsigned long long cta_total = 0;
-    (void)cta_exclusive_scan(sum, &cta_total);
+    (void)cta_exclusive_scan<kRangeThreads>(sum, &cta_total);
     __shared__ bool last;
     if (threadIdx.x == 0) {
         cta_sum[blockIdx.x] = cta_total;
@@ -130,7 +105,7 @@ __global__ void __launch_bounds__(kRangeThreads) range_rank_kernel(
     unsigned long long local = 0;
     for (int64_t g = lo; g < hi; ++g) local += __ldcg(cta_sum + g);
     unsigned long long total = 0;
-    unsigned long long run = cta_exclusive_scan(local, &total);
+    unsigned long long run = cta_exclusive_scan<kRangeThreads>(local, &total);
     for (int64_t g = lo; g < hi; ++g) {
         const unsigned long long v = __ldcg(cta_sum + g);
         cta_sum[g] = run;
@@ -155,7 +130,7 @@ __global__ void __launch_bounds__(kRangeThreads) range_offsets_kernel(const unsi
         local += c[k];
     }
     unsigned long long cta_total = 0;
-    unsigned long long run = cta_base[blockIdx.x] + cta_exclusive_scan(local, &cta_total);
+    unsigned long long run = cta_base[blockIdx.x] + cta_exclusive_scan<kRangeThreads>(local, &cta_total);
 #pragma unroll
     for (int k = 0; k < kRangesPerThread; ++k) {
         if (base + k < nranges) offsets[base + k] = (int64_t)run;

@@ -468,6 +468,7 @@ struct MultiSmem {
     const uint32_t *bits;
     const uint2 *table;
     const uint2 *dir;
+    const uint32_t *occ;   // kDict: "home slot occupied", folded to 2^mocc_log2 bits (may say occupied wrongly, never empty)
 };
 __device__ __forceinline__ uint32_t multi_probe(const uint32_t *bits, uint32_t h)
 {
@@ -484,11 +485,14 @@ __device__ __forceinline__ bool multi_any(const uint4 &w, uint32_t w4, uint32_t 
 // A word whose hash is flagged AND whose home slot of the exact table is occupied: walk the probe sequence and compare
 // the text with every pattern that has this gram at some residue.  Rare (about K / 128 of the flagged words), out of
 // line, all arguments in registers.  Returns the hit bits of the chunk (bit = start - (chunk_v - 3)).
+// kMulti's table has kMultiSlots slots; a dictionary's (kDict) has 2^mslots_log2, in shared or global memory.
+template <Filter F>
 __device__ __noinline__ uint32_t multi_word(const ScanArgs &A, const uint2 *table, const uint2 *dir, const uint8_t *blob,
                                             uint32_t h, int j, int64_t chunk_v, const uint8_t *vbase)
 {
+    const uint32_t lg = F == kMulti ? (uint32_t)kMultiSlotsLog2 : A.mslots_log2, mask = (1u << lg) - 1u;
     uint32_t hits = 0;
-    for (uint32_t slot = (h * kMultiSlotMul) >> (32 - kMultiSlotsLog2);; slot = (slot + 1) & (kMultiSlots - 1)) {
+    for (uint32_t slot = (h * kMultiSlotMul) >> (32 - lg);; slot = (slot + 1) & mask) {
         const uint2 e = table[slot];
         if (e.y == 0u) break;
         if (e.x != h) continue;
@@ -511,7 +515,9 @@ __device__ __noinline__ uint32_t multi_word(const ScanArgs &A, const uint2 *tabl
 }
 // Exact check of one 16-byte chunk (start positions c-3 .. c+12, c = chunk_v): returns the union hit mask and bumps the
 // per-pattern counters.  Every start position is examined by exactly one thread of the grid.  A false positive of the
-// bitmap dies here at ONE shared-memory load (its home slot in the exact table is empty), without a call.
+// bitmap dies here at ONE shared-memory load (its home slot in the exact table is empty), without a call; a dictionary
+// whose table is too large for shared memory asks the staged occupancy bits instead of the table.
+template <Filter F>
 __device__ __forceinline__ uint32_t multi_chunk(const ScanArgs &A, const MultiSmem &M, const uint8_t *blob, const uint4 &w, uint32_t w4,
                                                 uint32_t w5, int64_t chunk_v, const uint8_t *vbase)
 {
@@ -520,8 +526,15 @@ __device__ __forceinline__ uint32_t multi_chunk(const ScanArgs &A, const MultiSm
     uint32_t hits = 0;
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-        if ((multi_probe(M.bits, h[j]) & 1u) && M.table[(h[j] * kMultiSlotMul) >> (32 - kMultiSlotsLog2)].y != 0u)
-            hits |= multi_word(A, M.table, M.dir, blob, h[j], j, chunk_v, vbase);
+        if (!(multi_probe(M.bits, h[j]) & 1u)) continue;
+        bool home;
+        if constexpr (F == kMulti) {
+            home = M.table[(h[j] * kMultiSlotMul) >> (32 - kMultiSlotsLog2)].y != 0u;
+        } else {
+            const uint32_t b = ((h[j] * kMultiSlotMul) >> (32 - A.mslots_log2)) & ((1u << A.mocc_log2) - 1u);
+            home = (M.occ[b >> 5] >> (b & 31u)) & 1u;
+        }
+        if (home) hits |= multi_word<F>(A, M.table, M.dir, blob, h[j], j, chunk_v, vbase);
     }
     return hits;
 }
@@ -671,17 +684,26 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
 
     extern __shared__ __align__(128) uint8_t smem[];
     SmemCtl *ctl = reinterpret_cast<SmemCtl *>(smem);
-    uint8_t *stages = smem + kCtlBytes + (F == kMulti ? A.multi_smem : 0u);
+    uint8_t *stages = smem + kCtlBytes + (filter_is_set(F) ? A.multi_smem : 0u);
 
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
     const uint32_t S = A.stages;
-    // multi-pattern variant: the shared candidate table sits between the control block and the stages
+    // multi-pattern variant: the shared candidate table sits between the control block and the stages.  A dictionary
+    // keeps bitmap | occupancy bits | (table, when it is staged) there; its directory stays in global memory.
     MultiSmem M;
     M.bits = reinterpret_cast<const uint32_t *>(smem + kCtlBytes);
-    M.table = reinterpret_cast<const uint2 *>(smem + kCtlBytes + (size_t)kMultiBitmapWords * 4);
-    M.dir = reinterpret_cast<const uint2 *>(smem + kCtlBytes + (size_t)kMultiBitmapWords * 4 + (size_t)kMultiSlots * 8);
-    const uint8_t *mblob = (F == kMulti && A.multi_blob_smem) ? reinterpret_cast<const uint8_t *>(ctl->good) : A.g_mblob;
+    if (F == kDict) {
+        const size_t occ_off = (size_t)kMultiBitmapWords * 4;
+        M.occ = reinterpret_cast<const uint32_t *>(smem + kCtlBytes + occ_off);
+        M.table = A.mtable_smem ? reinterpret_cast<const uint2 *>(smem + kCtlBytes + occ_off + ((size_t)1 << A.mocc_log2) / 8) : A.g_mtable;
+        M.dir = A.g_mdir;
+    } else {
+        M.occ = nullptr;
+        M.table = reinterpret_cast<const uint2 *>(smem + kCtlBytes + (size_t)kMultiBitmapWords * 4);
+        M.dir = reinterpret_cast<const uint2 *>(smem + kCtlBytes + (size_t)kMultiBitmapWords * 4 + (size_t)kMultiSlots * 8);
+    }
+    const uint8_t *mblob = (filter_is_set(F) && A.multi_blob_smem) ? reinterpret_cast<const uint8_t *>(ctl->good) : A.g_mblob;
 
     // Fetches one tile (plus the 16 bytes in front of it and the halo behind it) into pipeline slot s.
     auto fetch_tile = [&](uint32_t tile, uint32_t s) {
@@ -743,6 +765,15 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
         for (int i = tid; i < NB; i += kThreads) dst[i] = b4[i];
         for (int i = tid; i < NT; i += kThreads) dst[NB + i] = t4[i];
         for (int i = tid; i < ND; i += kThreads) dst[NB + NT + i] = d4[i];
+    }
+    if (F == kDict) {   // the image puts bitmap, occupancy bits and table one behind the other, as they are staged
+        uint4 *dst = reinterpret_cast<uint4 *>(smem + kCtlBytes);
+        const uint4 *src = reinterpret_cast<const uint4 *>(A.g_mbits);
+        const uint32_t nvec = (uint32_t)(((size_t)kMultiBitmapWords * 4 + ((size_t)1 << A.mocc_log2) / 8 +
+                                          (A.mtable_smem ? ((size_t)8 << A.mslots_log2) : 0)) / 16);
+        for (uint32_t i = tid; i < nvec; i += kThreads) dst[i] = src[i];
+    }
+    if (filter_is_set(F)) {
         if (A.multi_blob_smem) {   // the patterns themselves ride in the good-suffix area of the control block (unused here)
             uint4 *bd = reinterpret_cast<uint4 *>(ctl->good);
             const uint4 *bs = reinterpret_cast<const uint4 *>(A.g_mblob);
@@ -813,7 +844,7 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
         const bool all_valid = tile_v0 + OFFS >= A.vmin && tile_v0 + (TILE - 1) + OFFS <= A.vmax;
 
         bool took_dense = false;
-        if constexpr (F != kShiftAnd && F != kMulti) {
+        if constexpr (F != kShiftAnd && !filter_is_set(F)) {
             if (dense_mode) {
                 const VerifyCtx vc{vbase, pat, rpat, bad, good, exact_filter, all_valid};
                 unsigned long long r;
@@ -849,18 +880,18 @@ __global__ void __launch_bounds__(kThreads, 2) scan_kernel(const __grid_constant
                     uint32_t w4[4];
                     load_segment(st + seg_off, lane, w, w4);
                     uint32_t w5[4] = {0u, 0u, 0u, 0u};
-                    if (F == kMulti && A.hmul2 != 0u) load_second_after(st + seg_off, lane, w, w5);
+                    if (filter_is_set(F) && A.hmul2 != 0u) load_second_after(st + seg_off, lane, w, w5);
                     bool any[4];
 #pragma unroll
                     for (int sl = 0; sl < 4; ++sl)
-                        any[sl] = F == kMulti ? multi_any(w[sl], w4[sl], w5[sl], A.hmul, A.hmul2, M.bits) : filter_any<F>(w[sl], w4[sl], A);
+                        any[sl] = filter_is_set(F) ? multi_any(w[sl], w4[sl], w5[sl], A.hmul, A.hmul2, M.bits) : filter_any<F>(w[sl], w4[sl], A);
                     const uint32_t vote = __ballot_sync(0xFFFFFFFFu, any[0] | any[1] | any[2] | any[3]);
                     if (vote) {  // warp-uniform and rare: the common path ends at this branch
-                        if (F == kMulti) {
+                        if (filter_is_set(F)) {
 #pragma unroll
                             for (int sl = 0; sl < 4; ++sl) {
                                 if (any[sl]) {
-                                    hm[sl] = multi_chunk(A, M, mblob, w[sl], w4[sl], w5[sl], seg_p0 + sl * 512 - OFFS, vbase);
+                                    hm[sl] = multi_chunk<F>(A, M, mblob, w[sl], w4[sl], w5[sl], seg_p0 + sl * 512 - OFFS, vbase);
                                     seg_hits += __popc(hm[sl]);
                                 }
                             }
@@ -1492,14 +1523,15 @@ static KernelRow kernels_of()
 {
     KernelRow r{};
     fill_row<F, false>(r.k[0]);
-    if constexpr (F != kMulti) fill_row<F, true>(r.k[1]);
+    if constexpr (!filter_is_set(F)) fill_row<F, true>(r.k[1]);
     return r;
 }
 static const void *scan_kernel_for(Filter filter, int tile, bool positions, bool fold)
 {
     static const KernelRow rows[] = {kernels_of<kQgramPerResidue>(), kernels_of<kQgram>(), kernels_of<kWindow4>(),
                                      kernels_of<kBytes1>(),          kernels_of<kBytes2>(), kernels_of<kBytes3>(),
-                                     kernels_of<kBytes5>(),          kernels_of<kShiftAnd>(), kernels_of<kMulti>()};
+                                     kernels_of<kBytes5>(),          kernels_of<kShiftAnd>(), kernels_of<kMulti>(),
+                                     kernels_of<kDict>()};
     static_assert(sizeof rows / sizeof rows[0] == kFilterCount, "one row per filter kind, in the order of enum Filter");
     return rows[filter].k[fold][tile == 32768][positions];
 }
@@ -1542,12 +1574,14 @@ int plan_scan(int device, Filter filter, bool fold, int32_t m, bool positions, S
     int sm_count = 0, smem_optin = 0, smem_sm = 0;
     if (int rc = device_info(device, &sm_count, &smem_optin, &smem_sm, nullptr)) return rc;
 
-    const bool multi = filter == kMulti;
+    const bool multi = filter_is_set(filter);
     // profiles/tune_knobs.py: 32 KiB tiles, 2 CTAs/SM, 3 stages.  The multi-pattern variant keeps 37 KiB of tables in
     // shared memory: 16 KiB tiles leave room for a 4-stage ring next to them.
     int tile = multi ? env_int("BMX_MULTI_TILE", 16384) : env_int("BMX_TILE", 32768);
     if (tile != 16384 && tile != 32768) tile = multi ? 16384 : 32768;
-    a->multi_smem = multi ? (uint32_t)((kMultiSmemBytes + 127) & ~size_t(127)) : 0u;
+    a->multi_smem = filter == kMulti  ? (uint32_t)((kMultiSmemBytes + 127) & ~size_t(127))
+                    : filter == kDict ? (uint32_t)dict_smem_bytes(a->mslots_log2, a->mtable_smem, a->mocc_log2)
+                                      : 0u;
     const int ctas_per_sm = std::max(1, std::min(2, env_int("BMX_CTAS_PER_SM", 2)));
 
     // Halo: enough for the filter's look-ahead (one more word; Shift-And reads 16+m-1 bytes per

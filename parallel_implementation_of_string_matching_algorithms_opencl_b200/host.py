@@ -391,6 +391,77 @@ class Scanner:
         return count.value, stats.as_dict()
 
 
+class Dictionary:
+    """A compiled pattern set for dictionary search (bmx_dict_*; `grep -F -f wordlist`): 1 .. 65536 patterns of
+    7 .. 4096 bytes each, hashed and uploaded once to `device`, then searched in one pass per text.
+
+    A match is a pair (p, k) with text[p:p+len(patterns[k])] == patterns[k]; the pairs come sorted by p, then k
+    (duplicate patterns are each reported).  counts[k] is exact and equals search(text, patterns[k])[0].  The
+    handle is immutable: several threads may search with it at once, each on its own stream.
+    """
+
+    def __init__(self, patterns, device: int = 0):
+        self._lib = _lib.load()
+        self._h = c_void_p()
+        pats = [_as_bytes(p) for p in patterns]
+        self.npat, self.device = len(pats), int(device)
+        self.min_length = min((len(p) for p in pats), default=0)
+        c_pats = (ctypes.c_char_p * self.npat)(*pats)
+        c_ms = (c_int32 * self.npat)(*[len(p) for p in pats])
+        check(self._lib.bmx_dict_create(self.device, self.npat, c_pats, c_ms, ctypes.byref(self._h)))
+
+    def close(self):
+        if self._h:
+            self._lib.bmx_dict_destroy(self._h)
+            self._h = c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def search(self, text, max_matches: int | None = None):
+        """HOST text (copied to the device once) -> (counts uint64[K], positions int64, pattern_ids int32, total).
+        positions / pattern_ids hold the first min(total, max_matches) pairs; None: room for all; 0: counts only."""
+        ptr, n, keep = _host_text(text)
+        counts = np.zeros(self.npat, dtype=np.uint64)
+        total = c_uint64(0)
+        open_ended = max_matches is None
+        cap = _first_cap(n, self.min_length) if open_ended else int(max_matches)
+        while True:
+            pos = np.empty(cap, dtype=np.int64)
+            pat = np.empty(cap, dtype=np.int32)
+            check(self._lib.bmx_dict_search(self._h, ptr, n, pos.ctypes.data if cap else None, pat.ctypes.data if cap else None,
+                                            cap, counts.ctypes.data, ctypes.byref(total)))
+            if not open_ended or total.value <= cap:
+                break
+            cap = int(total.value)
+        del keep
+        k = min(total.value, cap)
+        return counts, pos[:k], pat[:k], total.value
+
+    def search_device(self, text, max_matches: int = 0, pos_base: int = 0, stream=None):
+        """A contiguous CUDA uint8 tensor on the dictionary's device -> (counts uint64[K] on the host, positions int64
+        and pattern_ids int32 CUDA tensors holding the first min(total, max_matches) pairs or None, total).
+        Every position has pos_base added; max_matches=0 is counts only."""
+        import torch
+
+        _check_cuda(text, "uint8", "Dictionary.search_device(): text")
+        n, cap = text.numel(), int(max_matches)
+        counts = np.zeros(self.npat, dtype=np.uint64)
+        total = c_uint64(0)
+        with torch.cuda.device(text.device):
+            pos = torch.empty(cap, dtype=torch.int64, device=text.device) if cap else None
+            pat = torch.empty(cap, dtype=torch.int32, device=text.device) if cap else None
+            s = stream if stream is not None else torch.cuda.current_stream(text.device)
+            check(self._lib.bmx_dict_search_device(self._h, c_void_p(text.data_ptr() if n else 0), n, c_int64(pos_base),
+                                                   c_void_p(pos.data_ptr()) if cap else None, c_void_p(pat.data_ptr()) if cap else None,
+                                                   cap, counts.ctypes.data, ctypes.byref(total), c_void_p(s.cuda_stream)))
+        k = min(total.value, cap)
+        return counts, None if pos is None else pos[:k], None if pat is None else pat[:k], total.value
+
+
 class Exchange:
     """The exchange step of the sharded scan over NVLink peer memory (bmx_exchange_*): one per rank (= GPU).
 
